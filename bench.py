@@ -1,10 +1,14 @@
 #!/usr/bin/env python
 """bench.py -- the measurement contract of this repo.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4|cfg2|cfg3|cfg5|smallN] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4|cfg2|cfg3|cfg5|smallN] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
-One JSON line on rank 0.  A "step" is one MCMC step of every chain (one pass of the hot path over the batch).
+One JSON line on rank 0.  A "step" is one MCMC step of every chain (one pass of the hot path over the batch); the headline
+leg times exactly --steps of them, and `observed.grad_evals_per_chain_step` is the device's count of gradient evaluations
+in that timed run over chains x steps.
+--dump-outputs DIR writes what the timed run of the headline leg computed in its last step (rank 0's chains) as float64
+.npy files, so that two builds can be compared output for output: the inputs depend only on the arguments.
 
 Headline workload (BASELINE.json `metric` "chain-steps/s ..., HMC logistic regression", configs[3]):
   cfg4  HMCDA logistic regression, synthetic N = 1e6, d = 100 (X = [1, N(0,1)], beta0 ~ N(0,1)/sqrt(d), seed 4),
@@ -51,8 +55,8 @@ sys.path.insert(0, ROOT)
 # dual-averaged HMCDA step size after burn-in on cfg4 (median over 512 pilot chains; profiles/pilot_cfg4_r01.json)
 CFG4_EPS = 1.97e-3
 CFG4_LEN = 0.02
-CFG2_STEPS_PER_STEP = 200     # cfg2: MCMC steps per bench "step" (a single MCMC step of 65 536 3-D chains is ~2 us of work)
 ESS_SWEEP_LENS = (0.02, 0.008, 0.004)      # HMCDA trajectory lengths tried for min-ESS per gradient (10 / 4 / 2 leapfrogs)
+DUMP_BYTES = 64 * 10 ** 6 - 4096            # --dump-outputs writes at most 64 MB, .npy headers included
 
 
 def synth_logistic(N, d, seed):
@@ -89,11 +93,14 @@ WORKLOADS = {
                       "256 replicated chains, NCCL all-reduce of (d+2) x C partials per leapfrog (BASELINE configs[4])",
                  family="logistic", N=6250000, d=200, chains=256, sampler="HMC", seed=5),
     "cfg2": dict(desc="HMC(0.75) 3-D Normal -dot(v,v), 65536 chains/GPU (BASELINE configs[1])", family="normal_fn",
-                 N=0, d=3, chains=65536, sampler="HMC", seed=1),
+                 N=0, d=3, chains=65536, sampler="HMC", seed=1, steps=1000),
     "smallN": dict(desc="HMC (8 leapfrogs) logistic regression N=256 d=100, 94720 chains/GPU (5 full waves of 296 resident 64-chain CTAs): launch-bound small-N regime "
                         "(SURVEY 8d: 1e9 gradient evaluations/s is reachable only for N <~ 740)", family="logistic",
-                   N=256, d=100, chains=94720, sampler="HMC", seed=6, nleaps=8, eps=0.1),
+                   N=256, d=100, chains=94720, sampler="HMC", seed=6, nleaps=8, eps=0.1, steps=20),
 }
+# default --steps where a workload has none above: one MCMC step of cfg2 is ~2 us of device work and one of smallN ~3.4 ms, so
+# they time more steps by default to make the timed window long enough
+DEFAULT_STEPS = 5
 
 
 def config_block(name, wl, world):
@@ -169,6 +176,22 @@ def dgemm_peak_tflops(torch, n=8192, reps=5):
     del a, b, c
     torch.cuda.empty_cache()
     return 2.0 * n ** 3 / best / 1e9
+
+
+def dump_last_step(out_dir, res):
+    """--dump-outputs: the arrays fetch() returns for a run, at its last step (samples / grads (C, d), logtarget / accept (C,)).
+    When they exceed DUMP_BYTES, a fixed, seeded sample of chains is written; chain_index.npy lists the chains written."""
+    last = {k: np.asarray(v[:, -1], dtype=np.float64) for k, v in res.items()}
+    C = len(last["accept"])
+    per_chain = 8 * (1 + sum(v[0].size for v in last.values()))
+    idx = np.arange(C)
+    if C * per_chain > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(C, DUMP_BYTES // per_chain, replace=False))
+    out = {k: v[idx] for k, v in last.items()}
+    out["chain_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def make_problem(wl):
@@ -251,14 +274,10 @@ def run_reference_arm(args, wl, wl_name):
         return
     world = int(os.environ.get("WORLD_SIZE", "1"))
     cores = os.cpu_count() or 1
-    # bounded sample: steps sized so the run ends within a few minutes on the host cores
-    steps, warmup = args.steps, args.warmup
-    if wl_name in ("cfg2", "smallN"):
-        steps, warmup = max(steps, 1) * 2000, max(warmup, 1) * 200
-    cb = cpu_baseline(wl, steps, warmup, cores)
+    cb = cpu_baseline(wl, args.steps, args.warmup, cores)
     cfg = config_block(wl_name, wl, world)
     line = dict(metric="chain-steps/s", value=cb["value"], unit="chain-steps/s", n_gpus=args.gpus, steps=args.steps,
-                warmup=args.warmup, ms_per_step=1e3 * cb["seconds"] / steps, higher_is_better=True, scaling="weak",
+                warmup=args.warmup, ms_per_step=1e3 * cb["seconds"] / args.steps, higher_is_better=True, scaling="weak",
                 vs_baseline=None, dtype="f64", data="synthetic", impl="reference", config=cfg,
                 note="reference = CPU oracle (C restatement of MCMC.jl; the Julia 0.2 reference cannot run here), all host threads, "
                      "one chain per thread (the prun analogue); each step is one MCMC step of `cores` chains of the configured workload",
@@ -317,10 +336,18 @@ class Bench:
             self.peak = dgemm_peak_tflops(self.torch)
         return self.peak
 
+    def dump_run(self, r):
+        """--dump-outputs (rank 0): the last step of a timed run that has finished.  The C ABI returns a run's outputs only whole,
+        so every kept step of the samples and gradients crosses to the host here, once, after the timed region: 1.2 GB for
+        the smallN headline and 3.7 GB for cfg2 at their default --steps (as much as the e2e leg's pinned buffers)."""
+        if self.args.dump_outputs and self.rank == 0:
+            dump_last_step(self.args.dump_outputs, r.fetch(samples=True, grads=True, logtarget=True))
+
     # ---- one wave-engine leg: W warm-up steps, K timed steps of the same chains; returns device ms (this rank) ----
-    def wave_leg(self, dm, scfg, C, d, init_state, K, W, seed, offset, set_state=None, clock=False, time_eval=True):
+    def wave_leg(self, dm, scfg, C, d, init_state, K, W, seed, offset, set_state=None, clock=False, time_eval=True, dump=False):
         """time_eval: CUDA events around every likelihood launch (run_info.eval_ms / comm_ms); the engine then launches every
-        wave on the stream.  Without it the wave loop of the launch-bound workloads is replayed from a CUDA graph."""
+        wave on the stream.  Without it the wave loop of the launch-bound workloads is replayed from a CUDA graph.
+        dump: this is the headline leg, whose last step goes to --dump-outputs (after the timed region, see dump_run)."""
         capi, torch = self.capi, self.torch
         self.ctx.set_option("time_eval", 1 if time_eval else 0)
         step0 = set_state[0] if set_state else 0
@@ -339,6 +366,8 @@ class Bench:
             clk.__exit__()
         ms = e0.elapsed_time(e1)
         acc = float(r.fetch(samples=False, grads=False, logtarget=False)["accept"][:, W:].mean())
+        if dump:
+            self.dump_run(r)
         r.close()
         return ms, info, acc, (clk.summary() if clk else None)
 
@@ -432,7 +461,7 @@ def ess_pilot(B, dm, wl, init_state, set_state, offset, lens, ce=256, keep=400, 
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None, help="timed MCMC steps (default: 1000 for cfg2, 20 for smallN, else 5)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--workload", default="cfg4", choices=sorted(WORKLOADS))
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
@@ -443,8 +472,15 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="headline leg only (no configs / row_sharded / strong sub-blocks)")
     ap.add_argument("--cpu-steps", type=int, default=2)
     ap.add_argument("--shrink", type=int, default=1, help="divide the sizes of the sub-block workloads (tests)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
     wl = dict(WORKLOADS[args.workload])
+    if args.steps is None:
+        args.steps = wl.get("steps", DEFAULT_STEPS)
+    if args.steps < (2 if args.workload == "cfg2" and args.impl == "native" else 1):
+        ap.error("--steps must be at least 1 (2 for cfg2: its summaries leg takes batch means)")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the native arm's timed run")
     if args.chains:
         wl["chains"] = args.chains
     if args.N:
@@ -467,17 +503,18 @@ def main():
                 scaling="weak", vs_baseline=None, dtype="f64", data="synthetic", config=config_block(name, wl, world))
 
     if name == "cfg5":
-        blk = row_sharded_block(B, wl, K, W, parity=False)
+        blk = row_sharded_block(B, wl, K, W, parity=False, dump=True)
         line.update(value=blk["value"], ms_per_step=blk["ms_per_step"], gpu_launches=blk["gpu_launches"], e2e=blk["e2e"], clocks=blk.pop("clocks"),
                     roofline=blk["roofline"], row_sharded=blk)
     elif name == "cfg2":
-        blk = cfg2_block(B, wl, K, W, clock=True)
+        blk = cfg2_block(B, wl, K, W, clock=True, dump=True)
         line.update(value=blk["value"], ms_per_step=blk["ms"] / args.steps, gpu_launches=blk["gpu_launches"], e2e=blk["e2e"], clocks=blk["clocks"],
-                    roofline=blk["roofline"])
+                    roofline=blk["roofline"], observed=dict(grad_evals_per_chain_step=blk["grad_evals"] / (C * K)))
     elif name in ("cfg3", "smallN"):
-        blk = wave_block(B, name, wl, K if name == "cfg3" else 4 * K, W, clock=True)
+        blk = wave_block(B, name, wl, K, W, clock=True, dump=True)
         line.update(value=blk["value"], ms_per_step=blk["ms_per_step"], gpu_launches=blk["gpu_launches"], e2e=blk["e2e"], clocks=blk.pop("clocks"),
-                    roofline=blk["roofline"], grad_evals_per_s=blk["grad_evals_per_s"], observed=dict(accept_rate=blk["accept_rate"]))
+                    roofline=blk["roofline"], grad_evals_per_s=blk["grad_evals_per_s"],
+                    observed=dict(accept_rate=blk["accept_rate"], grad_evals_per_chain_step=blk["grad_evals"] / (C * K)))
     else:
         problem = make_problem(wl)
         X, y, hy, b0 = problem
@@ -486,7 +523,7 @@ def main():
         scfg = sampler_for(wl, capi)
         init_state, set_state = headline_state(wl, C, b0, rank)
         B.fp64_peak()
-        ms, info, acc_rate, clocks = B.wave_leg(dm, scfg, C, d, init_state, K, W, wl["seed"], offset, set_state, clock=True)
+        ms, info, acc_rate, clocks = B.wave_leg(dm, scfg, C, d, init_state, K, W, wl["seed"], offset, set_state, clock=True, dump=True)
         e2e_s, h2d, d2h = B.e2e_leg(dm, scfg, C, d, init_state, K, wl["seed"] + 1, offset, set_state)
         ms_max, e2e_ms_max = B.max_over_ranks(ms, e2e_s * 1e3)
         (evals,) = B.sum_over_ranks(float(info["n_grad_evals"]))
@@ -534,7 +571,7 @@ def main():
             w3 = dict(WORKLOADS["cfg3"]); w3["N"] //= sh; w3["chains"] //= sh
             cfgs["cfg3"] = wave_block(B, "cfg3", w3, 5, 3); cfgs["cfg3"].pop("clocks")
             w2 = dict(WORKLOADS["cfg2"]); w2["chains"] //= sh
-            cfgs["cfg2"] = cfg2_block(B, w2, 5, 3)
+            cfgs["cfg2"] = cfg2_block(B, w2, 1000, 600)
             ws = dict(WORKLOADS["smallN"]); ws["chains"] //= sh
             cfgs["smallN"] = wave_block(B, "smallN", ws, 20, 3); cfgs["smallN"].pop("clocks")
             line["configs"] = cfgs
@@ -550,7 +587,7 @@ def main():
         dist.destroy_process_group()
 
 
-def wave_block(B, name, wl, K, W, clock=False):
+def wave_block(B, name, wl, K, W, clock=False, dump=False):
     """compact sub-block: one regression workload through the wave engine (device-timed value, roofline, e2e)"""
     capi, world, rank = B.capi, B.world, B.rank
     C, d = wl["chains"], wl["d"]
@@ -560,7 +597,7 @@ def wave_block(B, name, wl, K, W, clock=False):
     scfg = sampler_for(wl, capi)
     init_state, set_state = headline_state(wl, C, b0, rank)
     # the value without per-launch events (graph replay of the wave loop), then the same steps with them for the kernel time
-    ms, info, acc, clocks = B.wave_leg(dm, scfg, C, d, init_state, K, W, wl["seed"], rank * C, set_state, clock=clock, time_eval=False)
+    ms, info, acc, clocks = B.wave_leg(dm, scfg, C, d, init_state, K, W, wl["seed"], rank * C, set_state, clock=clock, time_eval=False, dump=dump)
     ms_t, info_t, _, _ = B.wave_leg(dm, scfg, C, d, init_state, K, W, wl["seed"], rank * C, set_state, time_eval=True)
     B.ctx.set_option("time_eval", 0)
     e2e_s, h2d, d2h = B.e2e_leg(dm, scfg, C, d, init_state, K, wl["seed"] + 1, rank * C, set_state)
@@ -577,24 +614,24 @@ def wave_block(B, name, wl, K, W, clock=False):
     rf["share_of_step"] = info_t["eval_ms"] / ms                   # share of the (graph-replayed) step
     return dict(description=wl["desc"], N=wl["N"], d=d, chains_per_gpu=C, sampler=wl["sampler"], steps=K, warmup=W,
                 value=C * world * K / (ms_max / 1e3), unit="chain-steps/s", ms_per_step=ms_max / K,
-                grad_evals_per_s=evals / (ms_max / 1e3), accept_rate=acc, gpu_launches=int(info["n_launches"]), clocks=clocks, min_ess_per_s=ess,
+                grad_evals_per_s=evals / (ms_max / 1e3), grad_evals=int(info["n_grad_evals"]), accept_rate=acc, gpu_launches=int(info["n_launches"]),
+                clocks=clocks, min_ess_per_s=ess,
                 e2e=dict(value=C * world * K / (e2e_ms / 1e3), unit="chain-steps/s", h2d_bytes_per_step=h2d / K, d2h_bytes_per_step=d2h / K),
                 roofline=dict(bound="tensor", achieved=rf["achieved"], peak=rf["peak"], unit="TFLOP/s", frac=rf["frac"],
                               ms_per_launch=rf["ms_per_launch"], share_of_step=rf["share_of_step"]))
 
 
-def cfg2_block(B, wl, K, W, clock=False):
+def cfg2_block(B, wl, K, W, clock=False, dump=False):
     """fused per-chain kernel: the whole chain is one launch, so warm-up and timed region are separate runs"""
     capi, torch, world, rank = B.capi, B.torch, B.world, B.rank
     C, d = wl["chains"], wl["d"]
     dm = capi.DeviceModel(B.ctx, "normal_fn", d)
     scfg = sampler_for(wl, capi)
-    Ks, Ws = K * CFG2_STEPS_PER_STEP, W * CFG2_STEPS_PER_STEP
 
     def fresh(nsteps):
         return capi.DeviceRun(dm, scfg, (1, 1, nsteps), C, np.ones(d), seed=wl["seed"], chain_offset=rank * C, engine="fused")
-    r = fresh(Ws); r.execute(); r.close()
-    r = fresh(Ks)
+    r = fresh(W); r.execute(); r.close()
+    r = fresh(K)
     B.barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     clk = ClockSampler(B.local) if clock else None
@@ -605,15 +642,19 @@ def cfg2_block(B, wl, K, W, clock=False):
     if clk:
         clk.__exit__()
     ms = e0.elapsed_time(e1)
+    if dump:
+        B.dump_run(r)
     r.close()
-    e2e_s, h2d, d2h = B.e2e_leg(dm, scfg, C, d, np.ones(d), Ks, wl["seed"], rank * C, None, engine="fused")
+    e2e_s, h2d, d2h = B.e2e_leg(dm, scfg, C, d, np.ones(d), K, wl["seed"], rank * C, None, engine="fused")
     # summaries instead of draws: the same run, then src/stats on the device-resident draws (mean, MC variance, ESS, acceptance:
     # what ess(batch) / mean(batch) / acceptance(batch) of the host API do); only the d x C summaries cross PCIe
+    bl = min(100, K // 2)                # ess(vtype=:bm) needs at least two batches
     B.barrier()
     t0 = time.perf_counter()
-    r = capi.DeviceRun(dm, scfg, (1, 1, Ks), C, np.ones(d), seed=wl["seed"], chain_offset=rank * C, engine="fused", stream_stats=True)
+    r = capi.DeviceRun(dm, scfg, (1, 1, K), C, np.ones(d), seed=wl["seed"], chain_offset=rank * C, engine="fused", stream_stats=True,
+                       stream_batchlen=bl)
     r.execute()
-    st = r.stats("bm")
+    st = r.stats("bm", batchlen=bl)
     torch.cuda.synchronize()
     sum_s = time.perf_counter() - t0
     r.close()
@@ -622,14 +663,14 @@ def cfg2_block(B, wl, K, W, clock=False):
     bytes_per = 8 * d * 2 + 8 + 1       # sample + gradient + log-target + accept flag per kept chain-step
     pk = os.path.join(ROOT, "MEASURED_PEAKS.json")
     hbm = json.load(open(pk))["hbm_gbs"] if os.path.exists(pk) else 6650.0
-    ach = bytes_per * C * Ks / (ms / 1e3) / 1e9
-    return dict(description=wl["desc"], chains_per_gpu=C, steps=Ks, warmup=Ws, ms=ms_max, value=C * world * Ks / (ms_max / 1e3),
+    ach = bytes_per * C * K / (ms / 1e3) / 1e9
+    return dict(description=wl["desc"], chains_per_gpu=C, steps=K, warmup=W, ms=ms_max, grad_evals=int(info["n_grad_evals"]), value=C * world * K / (ms_max / 1e3),
                 unit="chain-steps/s", gpu_launches=int(info["n_launches"]), clocks=clk.summary() if clk else None,
-                e2e=dict(value=C * world * Ks / (e2e_ms / 1e3), unit="chain-steps/s", h2d_bytes_per_step=h2d / K, d2h_bytes_per_step=d2h / K),
-                e2e_summaries=dict(value=C * world * Ks / (sum_ms / 1e3), unit="chain-steps/s", h2d_bytes_per_step=d * 8 / K,
-                                   d2h_bytes_per_step=(5 * d + 1) * C * 8 / K, median_ess_per_step=float(np.median(st["ess"])) / Ks,
-                                   min_ess_per_s=float(np.median(st["ess"].min(axis=1))) / Ks * C * world * Ks / (ms_max / 1e3),
-                                   min_ess_note="median over chains of min over parameters of ess(vtype=:bm, batch length 100) per step x the device-timed chain-steps/s",
+                e2e=dict(value=C * world * K / (e2e_ms / 1e3), unit="chain-steps/s", h2d_bytes_per_step=h2d / K, d2h_bytes_per_step=d2h / K),
+                e2e_summaries=dict(value=C * world * K / (sum_ms / 1e3), unit="chain-steps/s", h2d_bytes_per_step=d * 8 / K,
+                                   d2h_bytes_per_step=(5 * d + 1) * C * 8 / K, median_ess_per_step=float(np.median(st["ess"])) / K,
+                                   min_ess_per_s=float(np.median(st["ess"].min(axis=1))) / K * C * world * K / (ms_max / 1e3),
+                                   min_ess_note=f"median over chains of min over parameters of ess(vtype=:bm, batch length {bl}) per step x the device-timed chain-steps/s",
                                    note="stream_stats run: mean / var_iid / var_bm / ess(bm) / actime / acceptance accumulated in registers while "
                                         "sampling (mcmcgpu_runner_cfg.stream_stats), no draw is stored; only the d x C summaries cross PCIe"),
                 roofline=dict(bound="hbm", achieved=ach, peak=hbm, unit="GB/s", frac=ach / hbm, traffic=None, kernel="fused_chain_kernel",
@@ -767,7 +808,7 @@ def population_block(B):
     return out
 
 
-def row_sharded_block(B, wl, K, W, parity):
+def row_sharded_block(B, wl, K, W, parity, dump=False):
     """cfg5: every rank generates ITS rows on the device (seeded per rank); chains replicated with identical Philox keys"""
     capi, torch, dist, world, rank = B.capi, B.torch, B.dist, B.world, B.rank
     d, C, N = wl["d"], wl["chains"], wl["N"]
@@ -791,7 +832,7 @@ def row_sharded_block(B, wl, K, W, parity):
     torch.cuda.empty_cache()
     scfg = sampler_for(wl, capi)
     init = b0[None, :] + 1e-3 * np.random.default_rng(100).standard_normal((C, d))   # same on every rank
-    ms, info, acc, clocks = B.wave_leg(dm, scfg, C, d, init, K, W, wl["seed"], 0, None, clock=True)
+    ms, info, acc, clocks = B.wave_leg(dm, scfg, C, d, init, K, W, wl["seed"], 0, None, clock=True, dump=dump)
     e2e_s, h2d, d2h = B.e2e_leg(dm, scfg, C, d, init, K, wl["seed"] + 1, 0, None)
     ms_max, e2e_ms, k1_ms, comm_ms = B.max_over_ranks(ms, e2e_s * 1e3, info["eval_ms"] / max(info["n_waves"], 1), info["comm_ms"] / max(info["n_waves"], 1))
     dm.close()

@@ -86,7 +86,8 @@ def test_out_of_support_semantics(O, capi, ctx):
     dm.close()
 
 
-def _run_both(O, capi, ctx, fam, d, X, y, hy, kind, skw, rngt, C, init, engine, scale=None, seed=1, force_eps=False):
+def _run_both(O, capi, ctx, fam, d, X, y, hy, kind, skw, rngt, C, init, engine, scale=None, seed=1, force_eps=False, chains=None):
+    """GPU run of C chains and oracle chains (all, or those listed in `chains`; None in refs for the others)"""
     om = O.Model(fam, d, X, y, hy)
     dm = capi.DeviceModel(ctx, fam, d, X, y, hy)
     rng = np.random.default_rng(seed)
@@ -96,13 +97,13 @@ def _run_both(O, capi, ctx, fam, d, X, y, hy, kind, skw, rngt, C, init, engine, 
     info = run.execute()
     out = run.fetch()
     diag = run.fetch_diag() if run.has_diag else None
-    refs = []
-    for c in range(C):
+    refs = [None] * C
+    for c in (range(C) if chains is None else chains):
         kw = dict(skw)
         if force_eps:
             kw["force_eps"] = np.concatenate([[np.nan], diag[0][c]])       # needs rngt = (1, 1, last)
         ini = init[c] if np.ndim(init) == 2 else init
-        refs.append(O.run_chain(om, O.sampler(kind, **kw), rngt, ini, scale, zn[c], un[c]))
+        refs[c] = O.run_chain(om, O.sampler(kind, **kw), rngt, ini, scale, zn[c], un[c])
     run.close(); dm.close()
     return out, diag, refs, info
 
@@ -933,21 +934,29 @@ def test_ram_large_d(O, capi, ctx, fam, d, N):
         capi.DeviceRun(capi.DeviceModel(ctx, "normal_dsl", 129, hyper=(0.0, 1.0)), capi.sampler_cfg("RAM", scale=1.0, rate=0.234), (1, 1, 5), 2, np.ones(129), engine="wave")
 
 
+_FUSED = [("HMC", dict(scale=0.02, nleaps=5), (11, 1, 60)),
+          ("HMC", dict(scale=0.02, nleaps=1), (1, 1, 40)),
+          ("HMC", dict(scale=0.02, nleaps=3, tuner=dict(target_rate=0.8, adapt_step=10)), (31, 2, 70)),
+          ("HMCDA", dict(len=0.1, max_leaps=64), (1, 1, 40)),
+          ("MALA", dict(scale=0.001), (1, 1, 40))]
+
+
 @pytest.mark.parametrize("fam", ["logistic", "probit", "linear"])
-@pytest.mark.parametrize("kind,skw,rngt", [("HMC", dict(scale=0.02, nleaps=5), (11, 1, 60)),
-                                           ("HMC", dict(scale=0.02, nleaps=1), (1, 1, 40)),
-                                           ("HMC", dict(scale=0.02, nleaps=3, tuner=dict(target_rate=0.8, adapt_step=10)), (31, 2, 70)),
-                                           ("HMCDA", dict(len=0.1, max_leaps=64), (1, 1, 40)),
-                                           ("MALA", dict(scale=0.001), (1, 1, 40))])
-def test_unsplit_likelihood_fuses_the_leapfrog(O, capi, ctx, fam, kind, skw, rngt):
+@pytest.mark.parametrize("kind,skw,rngt,d", [pytest.param(*c, 10, id=f"{c[0]}-skw{i}-rngt{i}") for i, c in enumerate(_FUSED)] +
+                         # fixed-length HMC at one d per resident-CTA class and probit table copy (DK 4, 8, 9, 13, 14, 25)
+                         [pytest.param(*_FUSED[0], d, id=f"HMC-skw0-rngt0-d{d}") for d in (29, 64, 71, 104, 112, 197)])
+def test_unsplit_likelihood_fuses_the_leapfrog(O, capi, ctx, fam, kind, skw, rngt, d):
     """one row split (the launch-bound small-N regime; forced here): the likelihood kernel makes the interior leapfrog
     updates and advances the chains' counters itself, the transition kernel is skipped on those waves (fixed-length HMC)
     or ignores those chains (HMCDA, tuned HMC).  Draw-matched against the oracle, stepwise == one call, evaluation counts."""
-    N, d, C = 700, 10, 70
+    N, C = 700, 70
     X, y, hy, _ = make_regression(fam, N, d, 6)
+    checked = range(C) if d == 10 else range(0, C, 5)   # oracle chains (CPU time grows with d)
     ctx.set_option("force_splits", 1)
     try:
         kw = dict(skw)
+        if "scale" in kw and d != 10:            # HMC's energy error grows with d and with X'X's condition number
+            kw["scale"] = kw["scale"] * math.sqrt(10 / d)
         if kind == "HMCDA":                      # realistic restored step sizes (the adaptation from eps = 1 is chaotic)
             rng = np.random.default_rng(1)
             eps = rng.uniform(0.01, 0.03, size=C)
@@ -960,13 +969,13 @@ def test_unsplit_likelihood_fuses_the_leapfrog(O, capi, ctx, fam, kind, skw, rng
             refs = [O.run_chain(om, O.sampler(kind, da_state=[eps[c], eps[c], 0.0], **kw), rngt, np.zeros(d), None, zn[c], un[c]) for c in range(C)]
             assert info["n_grad_evals"] == C + gnl.sum() and len(np.unique(gnl)) >= 3
         else:
-            out, diag, refs, info = _run_both(O, capi, ctx, fam, d, X, y, hy, kind, kw, rngt, C, np.zeros(d), "wave")
+            out, diag, refs, info = _run_both(O, capi, ctx, fam, d, X, y, hy, kind, kw, rngt, C, np.zeros(d), "wave", chains=checked)
             if kind == "HMC" and "tuner" not in kw:
                 assert info["n_grad_evals"] == C * (1 + rngt[2] * kw["nleaps"])
                 assert info["n_launches"] < 2 * info["n_waves"] or kw["nleaps"] == 1      # no transition launch on interior waves
         gs = np.abs(X).sum(0)
-        for c in range(C):
-            assert np.array_equal(refs[c]["accept"], out["accept"][c]), (fam, kind, c)
+        for c in checked:
+            assert np.array_equal(refs[c]["accept"], out["accept"][c]), (fam, kind, d, c)
             assert np.allclose(refs[c]["samples"], out["samples"][c], rtol=1e-9, atol=1e-12)
             assert np.allclose(refs[c]["logtarget"], out["logtarget"][c], rtol=1e-11, atol=0)
             assert np.all(np.abs(refs[c]["grads"] - out["grads"][c]) <= 1e-9 * gs)

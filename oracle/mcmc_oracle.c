@@ -374,6 +374,17 @@ static void store_kept(int64_t d, int64_t kept, const double* pp, double plt, co
   if (diag_nleaps) diag_nleaps[kept] = nl;
 }
 
+/* mean_rb_hmc, src/stats/mean.jl:17-31: (sample + sum_k exp(H0 - H_k) pars_k) / (nLeaps + 1) over the recorded leap
+ * states of one trajectory, written to rb_out[kept] */
+static void store_rb(double* rb_out, int64_t kept, int64_t d, const double* smp, double H0, const double* leapP,
+                     const double* leapH, int64_t nLeaps) {
+  for (int64_t jj = 0; jj < d; jj++) {
+    double sm = smp[jj];
+    for (int64_t k = 0; k < nLeaps; k++) sm += exp(H0 - leapH[k]) * leapP[k * d + jj];
+    rb_out[kept * d + jj] = sm / (double)(nLeaps + 1);
+  }
+}
+
 /* round() of Julia 0.2 == C round (half away from zero) (HMCDA.jl:104) */
 
 int32_t orc_run_chain(const orc_model* m, const orc_sampler* s, const orc_range* r,
@@ -483,12 +494,7 @@ int32_t orc_run_chain(const orc_model* m, const orc_sampler* s, const orc_range*
       }
       if (s->rb_out && in_range(i, r)) {                          /* mean_rb_hmc, src/stats/mean.jl:17-31 */
         int accn = uniforms[i] < exp(st0.H - st.H);
-        const double* smp = accn ? st.pars : st0.pars;            /* c.samples[i, :] */
-        for (int64_t jj = 0; jj < d; jj++) {
-          double sm = smp[jj];
-          for (int64_t k = 0; k < nLeaps; k++) sm += exp(st0.H - leapH[k]) * leapP[k * d + jj];
-          s->rb_out[kept * d + jj] = sm / (double)(nLeaps + 1);
-        }
+        store_rb(s->rb_out, kept, d, accn ? st.pars : st0.pars, st0.H, leapP, leapH, nLeaps);   /* c.samples[i, :] */
       }
       if (leapP) { free(leapP); free(leapH); }
       if (uniforms[i] < exp(st0.H - st.H)) {                      /* :154 */
@@ -546,11 +552,18 @@ int32_t orc_run_chain(const orc_model* m, const orc_sampler* s, const orc_range*
       if (!(nl >= 1.0)) nl = 1.0;                                 /* max(1, .) */
       if (s->max_leaps > 0 && nl > (double)s->max_leaps) nl = (double)s->max_leaps; /* documented cap */
       int64_t nLeaps = (int64_t)nl;
-      for (int64_t j = 0; j < nLeaps; j++) hs_leapfrog(&st, leapStep, m, &nev); /* :107-109 */
+      double* leapP = NULL; double* leapH = NULL;                 /* storeLeaps, as in the HMC branch */
+      if (s->rb_out) { leapP = (double*)malloc(sizeof(double) * (size_t)(nLeaps * d)); leapH = (double*)malloc(sizeof(double) * (size_t)nLeaps); }
+      for (int64_t j = 0; j < nLeaps; j++) {                      /* :107-109 */
+        hs_leapfrog(&st, leapStep, m, &nev);
+        if (s->rb_out) { memcpy(leapP + j * d, st.pars, sizeof(double) * (size_t)d); leapH[j] = st.H; }
+      }
       double e = exp(st0.H - st.H);
       /* p = min(1, exp(H0-H)) (:120).  Documented deviation: a NaN ratio is treated as p = 0
        * (reject, adapt with 0) instead of poisoning dualH/leapStep for the rest of the run. */
       double p = isnan(e) ? 0.0 : (e < 1.0 ? e : 1.0);
+      if (s->rb_out && in_range(i, r)) store_rb(s->rb_out, kept, d, uniforms[i] < p ? st.pars : st0.pars, st0.H, leapP, leapH, nLeaps);
+      if (leapP) { free(leapP); free(leapH); }
       double eps_used = own_eps;
       if (uniforms[i] < p) {                                      /* :121 */
         STORE(st.pars, st.logTarget, st.grad, 1, eps_used, nLeaps);

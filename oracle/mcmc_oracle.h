@@ -61,8 +61,9 @@ typedef struct {
    * bound over a burn-in.  When force_eps != NULL (length last+1) the trajectory of step i uses
    * force_eps[i] while diag_eps still reports the oracle's own adapted value: a one-step-ahead check. */
   const double* force_eps;
-  /* HMC storeLeaps (HMC.jl:145-150): when rb_out != NULL (S x d) the leap states are kept for the step and the
-   * Rao-Blackwell sums of mean_rb_hmc (src/stats/mean.jl:11-35) are written per kept step. */
+  /* HMC / HMCDA storeLeaps (HMC.jl:145-150): when rb_out != NULL (S x d) the leap states are kept for the step and the
+   * Rao-Blackwell sums of mean_rb_hmc (src/stats/mean.jl:11-35) are written per kept step; the sample they start from
+   * is the one the sampler's own acceptance test keeps (HMCDA: u < min(1, e)). */
   double* rb_out;
   /* test aid (not in the reference, whose resume restarts from model.init, SerialMC.jl:93-97): the chain starts at
    * step start_step + 1 from `init` (draw columns keep their absolute step index), and, for HMCDA, da_state != NULL

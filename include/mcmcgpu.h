@@ -50,6 +50,15 @@ extern "C" {
 #define MCMCGPU_HMC 2
 #define MCMCGPU_HMCDA 3
 #define MCMCGPU_RAM 4          /* src/samplers/RAM.jl:24-36: scale, rate (robust adaptive Metropolis); d <= 8 fused, d <= 128 wave */
+/* No-U-Turn sampler: slice NUTS with dual averaging (Hoffman & Gelman 2014, Algorithms 3 and 6), identity mass matrix,
+ * engine WAVE only (one leapfrog leaf per chain per wave).  It reads mcmcgpu_sampler_cfg as follows:
+ *   nleaps = maxdoublings (1..10: at most 2^maxdoublings - 1 leapfrogs per step);
+ *   rate, shrinkage, t0, step = the dual averaging, HMCDA's rules (the target is the mean acceptance statistic of the
+ *   last doubling); scale, len and max_leaps are ignored, and so is the model scale passed to the run.
+ * fetch_diag returns the step size and the leapfrog count of every kept step (ndoublings = floor(log2(leaps)) + 1);
+ * set_state / get_state carry (step size, dual step size, dualH) as for HMCDA.  Not supported: engine FUSED, injected
+ * draws, store_rb, a tuner, row-sharded models (MCMCGPU_E_ARG). */
+#define MCMCGPU_NUTS 5
 
 /* engines */
 #define MCMCGPU_ENGINE_AUTO 0
@@ -163,17 +172,17 @@ int32_t mcmcgpu_run_execute(mcmcgpu_run* run, mcmcgpu_run_info* info);
  * call continues exactly where the chains stopped (same Philox counters, same adaptation state). */
 int32_t mcmcgpu_run_execute_steps(mcmcgpu_run* run, int64_t nsteps, mcmcgpu_run_info* info);
 /* true resume (the reference's resume restarts from model.init, SerialMC.jl:93-97): before the first
- * execute, start the chains at step step0 + 1 (init = the saved positions) and, for HMCDA, restore the
+ * execute, start the chains at step step0 + 1 (init = the saved positions) and, for HMCDA / NUTS, restore the
  * dual-averaging state (arrays of nchains, or all NULL for the reference's initial values). */
 int32_t mcmcgpu_run_set_state(mcmcgpu_run* run, int64_t step0, const double* leapstep, const double* dual_leapstep,
                               const double* dualH);
-/* current positions (d x nchains) and HMCDA state (nchains each); any pointer may be NULL */
+/* current positions (d x nchains) and HMCDA / NUTS step-size state (nchains each); any pointer may be NULL */
 int32_t mcmcgpu_run_get_state(mcmcgpu_run* run, double* pars, double* leapstep, double* dual_leapstep, double* dualH);
 int32_t mcmcgpu_run_fetch(mcmcgpu_run* run, double* out_samples, double* out_grads, uint8_t* out_accept,
                           double* out_logtarget);
 /* Rao-Blackwellised draws (store_rb): out_rb d x S x nchains; their column means are mean_rb(chain) (mean.jl:37-41) */
 int32_t mcmcgpu_run_fetch_rb(mcmcgpu_run* run, double* out_rb);
-/* per-chain diagnostics: final leap step (HMCDA/tuned), kept-step leap steps (S x nchains) and leap counts */
+/* per-chain diagnostics: final leap step (HMCDA/NUTS/tuned), kept-step leap steps (S x nchains) and leap counts */
 int32_t mcmcgpu_run_fetch_diag(mcmcgpu_run* run, double* out_eps, int64_t* out_nleaps);
 /* src/stats on the device-resident draws: outputs d x nchains each (NULL = skip).
  * mean (mean.jl:6), var_iid (var.jl:7-8), var (vtype: var.jl:137-166), ess / actime (ess.jl:6-19),

@@ -10,12 +10,12 @@ INTEGRATION.md.  Everything that computes goes through the CUDA library: there i
     batch = run(m * HMCDA(len=0.02) * GPUMC(steps=400, burnin=200, nchains=10000))
     ess(batch), acceptance(chain), var(chain, vtype="bm")                 # src/stats
 """
-from .api import (EmpMCTuner, GPUMC, HMC, HMCDA, MALA, MCMCChain, MCMCChainBatch, MCMCLikelihoodModel, MCMCTask,
+from .api import (EmpMCTuner, GPUMC, HMC, HMCDA, MALA, NUTS, MCMCChain, MCMCChainBatch, MCMCLikelihoodModel, MCMCTask,
                   RAM, RWM, SerialMC, SeqMC, SerialTempMC, acceptance, actime, describe, linearZv, quadraticZv, ess, mean, mean_rb, model, prun, resume, run, std, var,
                   default_context, set_default_device, shard_rows, init_row_sharding, broadcast_unique_id)
 from ._capi import MCMCGPUError, LIB_PATH
 
-__all__ = ["model", "MCMCLikelihoodModel", "RWM", "RAM", "MALA", "HMC", "HMCDA", "EmpMCTuner", "SerialMC", "GPUMC", "SeqMC", "SerialTempMC",
+__all__ = ["model", "MCMCLikelihoodModel", "RWM", "RAM", "MALA", "HMC", "HMCDA", "NUTS", "EmpMCTuner", "SerialMC", "GPUMC", "SeqMC", "SerialTempMC",
            "MCMCTask", "MCMCChain", "MCMCChainBatch", "run", "prun", "resume", "mean", "mean_rb", "var", "std", "ess", "actime",
            "acceptance", "describe", "linearZv", "quadraticZv", "MCMCGPUError", "LIB_PATH", "default_context", "set_default_device", "shard_rows", "init_row_sharding",
            "broadcast_unique_id"]

@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("MCMCGPU_LIB") or os.path.join(_HERE, "libmcmcgpu.so")
 
 OK, E_ARG, E_SUPPORT, E_NOGRAD, E_CUDA, E_COMM, E_STATE = 0, -1, -2, -3, -4, -5, -6
 FAM = dict(normal_fn=0, normal_dsl=1, linear=2, logistic=3, probit=4, ou=5, abs_normal=6)
-KIND = dict(RWM=0, MALA=1, HMC=2, HMCDA=3, RAM=4)
+KIND = dict(RWM=0, MALA=1, HMC=2, HMCDA=3, RAM=4, NUTS=5)
 ENGINE = dict(auto=0, fused=1, wave=2)
 VTYPE = dict(iid=0, bm=1, imse=2, ipse=3)
 
@@ -360,7 +360,7 @@ class DeviceRun(_Owned):
         self.S = 0 if (step < 1 or last < first) else (last - first) // step + 1
         self.C = nchains
         self.store_grad, self.store_logtarget = store_grad, store_logtarget
-        self.has_diag = bool(scfg.kind in (KIND["HMCDA"], KIND["RAM"]) or scfg.tuner_on)
+        self.has_diag = bool(scfg.kind in (KIND["HMCDA"], KIND["RAM"], KIND["NUTS"]) or scfg.tuner_on)
         sc = None if scale is None else f64(np.broadcast_to(scale, (self.d,)).copy())
         zn = f64(normals)
         un = f64(uniforms)

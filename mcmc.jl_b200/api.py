@@ -299,6 +299,26 @@ class HMCDA(_Sampler):
                                 step=self.step, max_leaps=self.max_leaps)
 
 
+class NUTS(_Sampler):
+    """No-U-Turn sampler: slice NUTS with dual averaging of the step size (Hoffman & Gelman 2014, Algorithms 3 and 6),
+    identity mass matrix.  rate is the target mean acceptance statistic, maxdoublings caps the tree at
+    2^maxdoublings - 1 leapfrogs per step, shrinkage / t0 / step are the dual averaging's gamma / t0 / kappa (HMCDA's).
+    Runs on the wave engine; the model's scale is not used."""
+
+    def __init__(self, rate=0.6, maxdoublings=10, shrinkage=0.05, t0=10.0, step=0.75):
+        assert 0.0 < rate < 1.0, f"Target acceptance rate ({rate}) should be between 0 and 1"
+        assert isinstance(maxdoublings, (int, np.integer)) and 1 <= maxdoublings <= 10, \
+            f"maxdoublings parameter of NUTS sampler ({maxdoublings}) must be an integer in 1..10"
+        assert shrinkage > 0.0, f"shrinkage parameter of NUTS sampler ({shrinkage}) must be positive"
+        assert t0 >= 0, f"t0 parameter of NUTS sampler ({t0}) must be non-negative"
+        self.rate, self.maxdoublings, self.shrinkage, self.t0, self.step = rate, int(maxdoublings), shrinkage, t0, step
+        self.tuner = None
+
+    def _cfg(self):
+        return capi.sampler_cfg("NUTS", nleaps=self.maxdoublings, rate=self.rate, shrinkage=self.shrinkage, t0=self.t0,
+                                step=self.step)
+
+
 # ---------------------------------------------------------------------------------------------------
 # runners (src/runners)
 # ---------------------------------------------------------------------------------------------------
@@ -474,12 +494,22 @@ class MCMCChainBatch:
     def __getitem__(self, i):
         a = self.arrays()
         diags = {"step": np.array(list(self.range)), "accept": a["accept"][i].astype(bool)}
+        if isinstance(self.task.sampler, NUTS):
+            eps, leaps = self.diag()
+            diags["epsilon"] = eps[i]
+            diags["ndoublings"] = np.floor(np.log2(leaps[i])).astype(np.int64) + 1    # the tree of 2^(n-1) .. 2^n - 1 leapfrogs
         g = a.get("grads")
         return MCMCChain(self.range, a["samples"][i], None if g is None else g[i], diags, self.task, self.runTime,
                          _colnames(self.task.model))
 
     def __iter__(self):
         return (self[i] for i in range(self.nchains))
+
+    def diag(self):
+        """(C, S) step sizes and (C, S) leapfrog counts of the kept steps (HMCDA, NUTS, RAM, tuned samplers)"""
+        if getattr(self, "_diag", None) is None:
+            self._diag = self._run.fetch_diag()
+        return self._diag
 
     def stats(self, vtype="imse", **kw):
         return self._run.stats(vtype, kw.get("maxlag", -1), kw.get("batchlen", 100))
@@ -604,7 +634,7 @@ def _population_tasks(tasks):
     for t in tasks:
         if t.sampler.needs_gradient and not t.model.has_gradient:
             raise AssertionError(f"{type(t.sampler).__name__} sampler requires model with gradient function")
-        if getattr(t.sampler, "tuner", None) is not None or isinstance(t.sampler, HMCDA):
+        if getattr(t.sampler, "tuner", None) is not None or isinstance(t.sampler, (HMCDA, NUTS)):
             raise NotImplementedError("population runners take RWM, MALA or HMC tasks without tuner")
     return m0, [t.model.hyper for t in tasks], [t.sampler._cfg() for t in tasks]
 

@@ -158,6 +158,14 @@ __device__ __forceinline__ double philox_uniform(uint64_t seed, uint64_t chain, 
   u4 o = philox4x32_10((uint32_t)chain, (uint32_t)(chain >> 32), step, 0xFFFFFFFFu, (uint32_t)seed, (uint32_t)(seed >> 32));
   return u01(o.x, o.y);
 }
+// uniform of an arbitrary block of step `step`: NUTS draws its tree directions (blocks 0x80000000 + 2j), subtree merges
+// (0x80000000 + 2j + 1) and leaf candidates (0x40000000 + k) here; the normal blocks 0 .. (d-1)/2 and the Metropolis
+// block 0xFFFFFFFF stay apart from them
+__device__ __forceinline__ double philox_slot_uniform(uint64_t seed, uint64_t chain, uint32_t step, uint32_t block) {
+  u4 o = philox4x32_10((uint32_t)chain, (uint32_t)(chain >> 32), step, block, (uint32_t)seed, (uint32_t)(seed >> 32));
+  return u01(o.x, o.y);
+}
+constexpr uint32_t NUTS_LEAF_BLOCK = 0x40000000u, NUTS_TREE_BLOCK = 0x80000000u;
 
 // ---------------------------------------------------------------------------------------------
 // scalar log-densities (Distributions.jl 2013 == Rmath dnorm4 / dunif / pnorm log scale)

@@ -34,7 +34,7 @@ struct mcmcgpu_ctx {
   NcclComm comm = nullptr;
   int rank = 0, nranks = 1;
   int64_t time_eval = 0;      // option: time every likelihood launch with events
-  int64_t poll_every = 0;     // option: waves between completion polls (HMCDA / tuned HMC); 0 = automatic
+  int64_t poll_every = 0;     // option: waves between completion polls (HMCDA / NUTS / tuned HMC); 0 = automatic
   int64_t force_splits = 0;   // option: override K1 row splits
   int64_t k1_debug = 0;       // option (experiments): see K1Args::debug
   int64_t use_graphs = 1;     // option: replay fixed-length wave loops from a CUDA graph
@@ -106,6 +106,7 @@ struct mcmcgpu_run {
   int32_t *phase = nullptr, *leap = nullptr, *nleaps_cur = nullptr, *remaining = nullptr;
   int64_t *istep = nullptr, *kept = nullptr, *tn_nleaps = nullptr, *tn_acc = nullptr, *tn_prop = nullptr;
   uint8_t *need_ll = nullptr, *k1_done = nullptr;
+  NutsState nuts{};          // NUTS runs only
   int nsplit = 1;
   std::vector<void*> owned, owned_big;
   template <typename T>
@@ -448,6 +449,12 @@ static int check_cfg(const mcmcgpu_model* m, const mcmcgpu_sampler_cfg* s, const
       if (!(s->shrinkage > 0)) return fail(MCMCGPU_E_ARG, "shrinkage parameter of HMCDA sampler must be positive");
       if (!(s->t0 >= 0)) return fail(MCMCGPU_E_ARG, "t0 parameter of HMCDA sampler must be non-negative");
       break;
+    case MCMCGPU_NUTS:                                                                                            // HMCDA's rules
+      if (!(s->rate > 0 && s->rate < 1)) return fail(MCMCGPU_E_ARG, "Target acceptance rate should be between 0 and 1");
+      if (!(s->shrinkage > 0)) return fail(MCMCGPU_E_ARG, "shrinkage parameter of NUTS sampler must be positive");
+      if (!(s->t0 >= 0)) return fail(MCMCGPU_E_ARG, "t0 parameter of NUTS sampler must be non-negative");
+      if (s->nleaps < 1 || s->nleaps > NUTS_MAX_DOUBLINGS) return fail(MCMCGPU_E_ARG, "NUTS maxdoublings should be in 1..10");
+      break;
     default: return fail(MCMCGPU_E_ARG, "unknown sampler kind");
   }
   if (s->tuner_on) {
@@ -492,11 +499,19 @@ static int run_create_impl(mcmcgpu_model* m, const mcmcgpu_sampler_cfg* s, const
   R->C = C; R->Cp = Cp; R->S = S; R->d = d;
   int engine = r->engine;
   const bool can_fuse = fused_supported(m->family, d, m->N);
+  const bool nuts = s->kind == MCMCGPU_NUTS;
+  if (nuts) {
+    const char* why = engine == MCMCGPU_ENGINE_FUSED ? "NUTS runs on engine WAVE only (engine FUSED has no NUTS)"
+                      : inj_normals ? "NUTS draws its own Philox numbers: injected normals / uniforms are not supported"
+                      : r->store_rb ? "storeLeaps applies to HMC / HMCDA" : m->row_sharded ? "NUTS does not support row-sharded models" : nullptr;
+    if (why) { delete R; return fail(MCMCGPU_E_ARG, why); }
+    engine = MCMCGPU_ENGINE_WAVE;
+  }
   if (engine == MCMCGPU_ENGINE_AUTO) engine = can_fuse ? MCMCGPU_ENGINE_FUSED : MCMCGPU_ENGINE_WAVE;
   if (engine == MCMCGPU_ENGINE_FUSED && !can_fuse) { delete R; return fail(MCMCGPU_E_ARG, "engine FUSED supports the closed-form families with d <= 8"); }
   if (engine != MCMCGPU_ENGINE_FUSED && engine != MCMCGPU_ENGINE_WAVE) { delete R; return fail(MCMCGPU_E_ARG, "unknown engine"); }
   R->engine = engine;
-  R->has_diag = (s->kind == MCMCGPU_HMCDA) || (s->kind == MCMCGPU_RAM) || s->tuner_on;
+  R->has_diag = (s->kind == MCMCGPU_HMCDA) || (s->kind == MCMCGPU_RAM) || nuts || s->tuner_on;
   if (s->kind == MCMCGPU_RAM && engine == MCMCGPU_ENGINE_WAVE && d > RAM_BIG_MAX_D) { delete R; return fail(MCMCGPU_E_ARG, "RAM supports d <= 128"); }
 #define RCU(x) do { cudaError_t e__ = (x); if (e__ != cudaSuccess) { std::string msg = std::string("CUDA: ") + cudaGetErrorString(e__) + " at " + __FILE__ + ":" + std::to_string(__LINE__); mcmcgpu_run_destroy(R); return fail(MCMCGPU_E_CUDA, msg); } } while (0)
   // inputs
@@ -597,6 +612,28 @@ static int run_create_impl(mcmcgpu_model* m, const mcmcgpu_sampler_cfg* s, const
       RCU(R->alloc(&R->ram_al, (size_t)Cp));
       RCU(R->alloc(&R->ram_pending, (size_t)Cp));
     }
+    if (nuts) {      // (8 + 2 (maxdoublings - 1)) d doubles and 10 scalars per chain
+      NutsState& T = R->nuts;
+      for (int sd = 0; sd < 2; sd++) {
+        RCU(R->alloc(&T.th[sd], (size_t)(d * Cp), false));
+        RCU(R->alloc(&T.p[sd], (size_t)(d * Cp), false));
+        RCU(R->alloc(&T.g[sd], (size_t)(d * Cp), false));
+      }
+      RCU(R->alloc(&T.sub_pars, (size_t)(d * Cp), false));
+      RCU(R->alloc(&T.sub_grad, (size_t)(d * Cp), false));
+      RCU(R->alloc(&T.sub_lt, (size_t)Cp));
+      RCU(R->alloc(&T.ck_th, (size_t)((s->nleaps - 1) * d * Cp), false));
+      RCU(R->alloc(&T.ck_p, (size_t)((s->nleaps - 1) * d * Cp), false));
+      RCU(R->alloc(&T.log_u0, (size_t)Cp));
+      RCU(R->alloc(&T.alpha, (size_t)Cp));
+      RCU(R->alloc(&T.j, (size_t)Cp));
+      RCU(R->alloc(&T.leaf, (size_t)Cp));
+      RCU(R->alloc(&T.leaps, (size_t)Cp));
+      RCU(R->alloc(&T.n, (size_t)Cp));
+      RCU(R->alloc(&T.n_sub, (size_t)Cp));
+      RCU(R->alloc(&T.dir, (size_t)Cp));
+      RCU(R->alloc(&T.moved, (size_t)Cp));
+    }
   }
   RCU(cudaStreamSynchronize(st));
   *out = R;
@@ -693,11 +730,11 @@ static int execute_impl(mcmcgpu_run* R, int64_t nsteps, mcmcgpu_run_info* info) 
     W.init = R->init; W.scale = R->scale; W.inj_normals = R->inj_normals; W.inj_uniforms = R->inj_uniforms;
     W.samples = R->samples; W.grads = R->grads; W.accept = R->accept; W.logtarget = R->logtarget;
     W.eps = R->eps; W.nleaps = R->nleaps; W.final_eps = R->final_eps; W.rb = R->rb; W.rb_acc = R->rb_acc;
-    W.init_lt = R->init_lt; W.chain_ids = R->chain_ids;
+    W.init_lt = R->init_lt; W.chain_ids = R->chain_ids; W.nuts = R->nuts;
     const int kind = R->s.kind;
     const bool need_grad = (kind != MCMCGPU_RWM && kind != MCMCGPU_RAM);
     const bool is_ram = (kind == MCMCGPU_RAM);
-    // RWM / MALA / RAM: every chain needs the log-target on every wave -- tell the likelihood kernel so (null flag array)
+    // RWM / MALA / RAM / NUTS: every chain needs the log-target on every wave -- tell the likelihood kernel so (null flag array)
     const uint8_t* need_ll_flags = (kind == MCMCGPU_HMC || kind == MCMCGPU_HMCDA) ? R->need_ll : nullptr;
     // number of waves when it is known in advance; otherwise poll the device counter
     int64_t known = -1;
@@ -853,7 +890,7 @@ int32_t mcmcgpu_run_set_state(mcmcgpu_run* R, int64_t step0, const double* leaps
   CU(use_ctx(R->m->ctx));
   R->step0 = step0;
   if (leapstep || dual_leapstep || dualH) {
-    if (R->s.kind != MCMCGPU_HMCDA) return fail(MCMCGPU_E_ARG, "step-size state applies to HMCDA");
+    if (R->s.kind != MCMCGPU_HMCDA && R->s.kind != MCMCGPU_NUTS) return fail(MCMCGPU_E_ARG, "step-size state applies to HMCDA and NUTS");
     if (!leapstep || !dual_leapstep || !dualH) return fail(MCMCGPU_E_ARG, "give leapstep, dual_leapstep and dualH together");
     int rc;
     if ((rc = upload_chain_vec(R, R->da_leapstep, leapstep))) return rc;

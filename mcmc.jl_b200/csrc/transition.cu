@@ -97,6 +97,36 @@ __device__ __forceinline__ double fin_grad(const EvalFin& f, const ModelDev& M, 
   return part[j * Cp + c];
 }
 
+// Keeps chain c's current state as the draw of step `step` when the step is in first:step:last.
+__device__ __forceinline__ void store_kept(const WaveArgs& W, const int64_t c, int64_t step, bool has_grad, bool acc, double eps, int nl) {
+  const RunnerDev& R = W.R;
+  const int64_t d = W.M.d, Cp = R.Cp;
+  // SerialMC.jl:49-66: the post-decision state (ppars / plogtarget / pgrads) is what is kept
+  if (!in_range(step, R.first, R.step, R.last)) return;
+  int64_t k = W.kept[c];
+  for (int64_t j = 0; j < d; j++) W.samples[(k * d + j) * Cp + c] = W.cur_pars[j * Cp + c];
+  if (W.grads) for (int64_t j = 0; j < d; j++) W.grads[(k * d + j) * Cp + c] = has_grad ? W.cur_grad[j * Cp + c] : CUDART_NAN;
+  W.accept[k * Cp + c] = acc ? 1 : 0;
+  if (W.logtarget) W.logtarget[k * Cp + c] = W.cur_lt[c];
+  if (W.eps) W.eps[k * Cp + c] = eps;
+  if (W.nleaps) W.nleaps[k * Cp + c] = nl;
+  W.kept[c] = k + 1;
+}
+
+// The dual-averaging update of step i < burnin (HMCDA.jl:133-138), shared by HMCDA (pacc = its acceptance probability)
+// and NUTS (pacc = the mean acceptance statistic of the step's last doubling).
+struct DaStep { double leapstep, dual, dualH; };
+__device__ __forceinline__ DaStep da_adapt(const SamplerDev& S, int64_t i, double pacc, double dual, double dualH) {
+  const double fi = (double)i;
+  double eta = 1.0 / (fi + S.t0);
+  DaStep r;
+  r.dualH = (1.0 - eta) * dualH + eta * (S.rate - pacc);
+  r.leapstep = exp(log(10.0 * 1.0) - sqrt(fi) * r.dualH / S.shrinkage);   // mu = log(10*leapStep0), leapStep0 = 1
+  eta = pow(fi, -S.step);
+  r.dual = exp((1.0 - eta) * log(dual) + eta * log(r.leapstep));
+  return r;
+}
+
 // One chain's share of a wave.  Returns the number of evaluations it consumed (0 or 1).  `interior_done`: the chain is in the
 // middle of a trajectory and its momentum / position update has already been made element-parallel by the caller
 // (transition_kernel, stage A); only the per-chain counters are left.
@@ -132,18 +162,7 @@ __device__ int transition_chain(const WaveArgs& W, const int64_t c, const bool i
   auto uniform = [&](int64_t step) -> double {
     return W.inj_uniforms ? W.inj_uniforms[step * Cp + c] : philox_uniform(R.seed, gchain, (uint32_t)step);
   };
-  auto store = [&](int64_t step, bool has_grad, bool acc, double eps, int nl) {
-    // SerialMC.jl:49-66: the post-decision state (ppars / plogtarget / pgrads) is what is kept
-    if (!in_range(step, R.first, R.step, R.last)) return;
-    int64_t k = W.kept[c];
-    for (int64_t j = 0; j < d; j++) W.samples[(k * d + j) * Cp + c] = W.cur_pars[j * Cp + c];
-    if (W.grads) for (int64_t j = 0; j < d; j++) W.grads[(k * d + j) * Cp + c] = has_grad ? W.cur_grad[j * Cp + c] : CUDART_NAN;
-    W.accept[k * Cp + c] = acc ? 1 : 0;
-    if (W.logtarget) W.logtarget[k * Cp + c] = W.cur_lt[c];
-    if (W.eps) W.eps[k * Cp + c] = eps;
-    if (W.nleaps) W.nleaps[k * Cp + c] = nl;
-    W.kept[c] = k + 1;
-  };
+  auto store = [&](int64_t step, bool has_grad, bool acc, double eps, int nl) { store_kept(W, c, step, has_grad, acc, eps, nl); };
 
   if (ph == PH_PAUSE) {
     begin = true;
@@ -271,13 +290,8 @@ __device__ int transition_chain(const WaveArgs& W, const int64_t c, const bool i
     store(i, true, acc, eps, nl_cur);
     if (kind == MCMCGPU_HMCDA) {
       if (i < burnin) {                                               // HMCDA.jl:133-138
-        double fi = (double)i;
-        double eta = 1.0 / (fi + S.t0);
-        double dualH = (1.0 - eta) * W.da_dualH[c] + eta * (S.rate - pacc);
-        double ls = exp(log(10.0 * 1.0) - sqrt(fi) * dualH / S.shrinkage);   // mu = log(10*leapStep0), leapStep0 = 1
-        eta = pow(fi, -S.step);
-        W.da_dual[c] = exp((1.0 - eta) * log(W.da_dual[c]) + eta * log(ls));
-        W.da_dualH[c] = dualH; W.da_leapstep[c] = ls;
+        const DaStep a = da_adapt(S, i, pacc, W.da_dual[c], W.da_dualH[c]);
+        W.da_dual[c] = a.dual; W.da_dualH[c] = a.dualH; W.da_leapstep[c] = a.leapstep;
       } else {
         W.da_leapstep[c] = W.da_dual[c];                              // :140
       }
@@ -639,13 +653,8 @@ __global__ void __launch_bounds__(CO_CHAINS * CO_GROUPS, 2) transition_coop_kern
         stored = true; st_eps = eps_cur; st_nl = nlc;
         if (kind == MCMCGPU_HMCDA) {
           if (i < burnin) {                                               // HMCDA.jl:133-138
-            const double fi = (double)i;
-            double eta = 1.0 / (fi + S.t0);
-            const double dualH = (1.0 - eta) * da_dualH_ld + eta * (S.rate - pacc);
-            const double ls = exp(log(10.0 * 1.0) - sqrt(fi) * dualH / S.shrinkage);
-            eta = pow(fi, -S.step);
-            W.da_dual[c] = exp((1.0 - eta) * log(da_dual_ld) + eta * log(ls));
-            W.da_dualH[c] = dualH; W.da_leapstep[c] = ls; da_ls_ld = ls;
+            const DaStep a = da_adapt(S, i, pacc, da_dual_ld, da_dualH_ld);
+            W.da_dual[c] = a.dual; W.da_dualH[c] = a.dualH; W.da_leapstep[c] = a.leapstep; da_ls_ld = a.leapstep;
           } else {
             W.da_leapstep[c] = da_dual_ld; da_ls_ld = da_dual_ld;         // :140
           }
@@ -793,7 +802,214 @@ __global__ void __launch_bounds__(CO_CHAINS * CO_GROUPS, 2) transition_coop_kern
   if (threadIdx.x == 0 && total) atomicAdd(W.n_evals, (unsigned long long)total);
 }
 
+// ---- NUTS: slice NUTS with dual averaging (Hoffman & Gelman 2014, Algorithms 3 and 6), one tree leaf per wave ----------
+// The recursion of BuildTree is unrolled into a per-chain state machine: doubling j builds a subtree of 2^j leaves from the
+// tree end on side v, one leapfrog (one evaluation) per leaf.  Leaf m of the subtree (1-based) leaves its (theta, p) in
+// checkpoint r for every r with (m - 1) mod 2^r == 0 -- the first leaf of every aligned 2^r-leaf block it opens -- and on
+// completion runs the U-turn check of every block it closes (m mod 2^r == 0), which is exactly the set of checks the
+// recursion makes.  Draws of step i: momentum from the normal blocks, slice uniform u0 from block 0xFFFFFFFF, direction
+// of doubling j from NUTS_TREE_BLOCK + 2j, its merge from NUTS_TREE_BLOCK + 2j + 1, candidate choice of the step's leaf
+// k (0-based) from NUTS_LEAF_BLOCK + k.  One thread per chain; every array is chain-minor, so a warp's accesses coalesce.
+
+// continue (true) unless a U-turn: delta = v (theta_m - theta_s), delta . p_s >= 0 and delta . p_m >= 0, summed in j order
+__device__ __forceinline__ bool nuts_no_uturn(const double* th_m, const double* p_m, const double* th_s, const double* p_s, double v,
+                                              int64_t d, int64_t Cp, int64_t c) {
+  double ds = 0.0, dm = 0.0;
+  for (int64_t j = 0; j < d; j++) {
+    const double delta = v * (th_m[j * Cp + c] - th_s[j * Cp + c]);
+    ds += delta * p_s[j * Cp + c];
+    dm += delta * p_m[j * Cp + c];
+  }
+  return ds >= 0.0 && dm >= 0.0;
+}
+
+__device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
+  const RunnerDev& R = W.R;
+  const SamplerDev& S = W.S;
+  const ModelDev& M = W.M;
+  const NutsState& T = W.nuts;
+  const int ph = W.phase[c];
+  if (ph == PH_DONE) return 0;
+  if (W.resume) {
+    if (ph != PH_PAUSE) return 0;
+    atomicAdd(W.remaining, 1);
+  } else if (ph == PH_PAUSE) return 0;
+  const int64_t d = M.d, Cp = R.Cp;
+  const uint64_t gchain = W.chain_ids ? (uint64_t)W.chain_ids[c] : (uint64_t)(R.chain_offset + c);
+  const int64_t burnin = R.first - 1;
+  double* q = W.q;
+  const double* part = W.part;
+  const int ns = W.nsplit;
+  int64_t i = W.istep[c];
+  int nev = 0;
+  EvalFin F; F.lt = CUDART_NAN; F.oos = false; F.ginv = 0.0; F.fam = M.family;
+  if (ph != PH_PAUSE) { F = finalize_eval(M, q, part, ns, Cp, c, true); nev = 1; }
+  bool begin = false, doubling = false;
+  int jnext = 0;
+
+  if (ph == PH_PAUSE) {
+    begin = true;
+  } else if (ph == PH_INIT) {
+    if (!isfinite(F.lt)) {   // "Initial values out of model support"
+      W.status[c] = 1; W.phase[c] = PH_DONE; atomicSub(W.remaining, 1);
+      return nev;
+    }
+    W.status[c] = 0;
+    W.cur_lt[c] = F.lt;
+    if (W.init_lt) W.init_lt[c] = F.lt;
+    for (int64_t j = 0; j < d; j++) {
+      W.cur_pars[j * Cp + c] = q[j * Cp + c];
+      W.cur_grad[j * Cp + c] = fin_grad(F, M, q, part, ns, Cp, c, j);
+    }
+    if (!W.restore_da) { W.da_leapstep[c] = 1.0; W.da_dual[c] = 1.0; W.da_dualH[c] = 0.0; }   // eps0 = 1, as HMCDA
+    i = W.step0 + 1;
+    begin = true;
+  } else {   // PH_NUTS: leaf `leaf` of the subtree of doubling jd has been evaluated at q
+    const int jd = T.j[c], side = T.dir[c], leaf = T.leaf[c];
+    const double v = side ? 1.0 : -1.0;
+    const double e = v * W.eps_cur[c];
+    double* th_v = T.th[side];
+    double* p_v = T.p[side];
+    double* g_v = T.g[side];
+    // end of the leapfrog (HMC.jl:98); the leaf becomes the tree's end on side v
+    double mm = 0.0;
+    for (int64_t j = 0; j < d; j++) {
+      const double gj = fin_grad(F, M, q, part, ns, Cp, c, j);
+      double m = W.mom[j * Cp + c];
+      m += (0.5 * gj) * e;
+      mm += m * m;
+      th_v[j * Cp + c] = q[j * Cp + c]; p_v[j * Cp + c] = m; g_v[j * Cp + c] = gj;
+    }
+    const double H = -F.lt + 0.5 * mm;                                  // update! HMC.jl:91
+    const double H0 = W.H0[c], lu0 = T.log_u0[c];
+    const int k = T.leaps[c];
+    T.leaps[c] = k + 1;
+    const double ea = exp(H0 - H);
+    const double alpha = T.alpha[c] + (isnan(ea) ? 0.0 : (ea < 1.0 ? ea : 1.0));
+    T.alpha[c] = alpha;
+    bool s = H - H0 < 1000.0 - lu0;                                     // false for NaN
+    if (lu0 <= H0 - H) {                                                // a valid leaf: candidate with probability 1 / n_sub
+      const int nsub = T.n_sub[c] + 1;
+      T.n_sub[c] = nsub;
+      if (nsub == 1 || philox_slot_uniform(R.seed, gchain, (uint32_t)i, NUTS_LEAF_BLOCK + (uint32_t)k) * (double)nsub < 1.0) {
+        for (int64_t j = 0; j < d; j++) { T.sub_pars[j * Cp + c] = th_v[j * Cp + c]; T.sub_grad[j * Cp + c] = g_v[j * Cp + c]; }
+        T.sub_lt[c] = F.lt;
+      }
+    }
+    const int64_t slot = d * Cp;
+    for (int r = 1; s && r <= jd && (leaf & ((1 << r) - 1)) == 0; r++)        // U-turn checks of the blocks this leaf closes
+      s = nuts_no_uturn(th_v, p_v, T.ck_th + (r - 1) * slot, T.ck_p + (r - 1) * slot, v, d, Cp, c);
+    bool open = false;
+    if (s && leaf < (1 << jd)) {                                        // next leaf of this subtree
+      for (int r = 1; r <= jd && ((leaf - 1) & ((1 << r) - 1)) == 0; r++)     // checkpoints of the blocks this leaf opens
+        for (int64_t j = 0; j < d; j++) {
+          T.ck_th[(r - 1) * slot + j * Cp + c] = th_v[j * Cp + c];
+          T.ck_p[(r - 1) * slot + j * Cp + c] = p_v[j * Cp + c];
+        }
+      for (int64_t j = 0; j < d; j++) {                                 // HMC.jl:95-96 from the end just reached
+        double m = p_v[j * Cp + c];
+        m += (0.5 * g_v[j * Cp + c]) * e;
+        double p = th_v[j * Cp + c];
+        p += e * m;
+        W.mom[j * Cp + c] = m; q[j * Cp + c] = p;
+      }
+      T.leaf[c] = leaf + 1;
+      return nev;
+    } else if (s) {                                                     // the subtree is complete: merge it into the tree
+      const int n = T.n[c], nsub = T.n_sub[c];
+      if (philox_slot_uniform(R.seed, gchain, (uint32_t)i, NUTS_TREE_BLOCK + 2u * (uint32_t)jd + 1u) * (double)n < (double)nsub) {
+        for (int64_t j = 0; j < d; j++) { W.cur_pars[j * Cp + c] = T.sub_pars[j * Cp + c]; W.cur_grad[j * Cp + c] = T.sub_grad[j * Cp + c]; }
+        W.cur_lt[c] = T.sub_lt[c];
+        T.moved[c] = 1;
+      }
+      T.n[c] = n + nsub;
+      open = jd + 1 < S.nleaps && nuts_no_uturn(T.th[1], T.p[1], T.th[0], T.p[0], 1.0, d, Cp, c);
+    }
+    if (open) {
+      doubling = true; jnext = jd + 1;
+    } else {                                                            // the tree is closed: the step's sample is final
+      const double pacc = alpha / (double)leaf;                         // alpha / n_alpha of the last doubling
+      store_kept(W, c, i, true, T.moved[c] != 0, W.eps_cur[c], k + 1);
+      if (i < burnin) {
+        const DaStep a = da_adapt(S, i, pacc, W.da_dual[c], W.da_dualH[c]);
+        W.da_dual[c] = a.dual; W.da_dualH[c] = a.dualH; W.da_leapstep[c] = a.leapstep;
+      } else {
+        W.da_leapstep[c] = W.da_dual[c];
+      }
+      i++; begin = true;
+    }
+  }
+
+  if (begin) {
+    W.istep[c] = i;
+    if (i > R.last) {
+      W.phase[c] = PH_DONE;
+      if (W.final_eps) W.final_eps[c] = W.da_leapstep[c];
+      atomicSub(W.remaining, 1);
+      return nev;
+    }
+    if (i > W.step_limit) {   // pause: mcmcgpu_run_execute_steps continues from here
+      W.phase[c] = PH_PAUSE;
+      atomicSub(W.remaining, 1);
+      return nev;
+    }
+    // ---- start step i: momentum, H0, slice, a one-point tree at the current state ----
+    double mm = 0.0;
+    for (int64_t jb = 0; jb < d; jb += 2) {
+      double z0, z1;
+      philox_normal_pair(R.seed, gchain, (uint32_t)i, (uint32_t)(jb >> 1), z0, z1);
+#pragma unroll
+      for (int t = 0; t < 2; t++) {
+        const int64_t j = jb + t;
+        if (j >= d) break;
+        const double z = t ? z1 : z0;
+        mm += z * z;
+        const double pj = W.cur_pars[j * Cp + c], gj = W.cur_grad[j * Cp + c];
+        T.th[0][j * Cp + c] = pj; T.th[1][j * Cp + c] = pj;
+        T.p[0][j * Cp + c] = z; T.p[1][j * Cp + c] = z;
+        T.g[0][j * Cp + c] = gj; T.g[1][j * Cp + c] = gj;
+      }
+    }
+    W.H0[c] = -W.cur_lt[c] + 0.5 * mm;                                  // update! HMC.jl:91
+    T.log_u0[c] = log(philox_uniform(R.seed, gchain, (uint32_t)i));
+    T.n[c] = 1; T.leaps[c] = 0; T.moved[c] = 0;
+    W.eps_cur[c] = W.da_leapstep[c];
+    doubling = true; jnext = 0;
+  }
+  if (doubling) {   // doubling jnext: direction, then the first leaf of its subtree from the end on that side
+    const int side = philox_slot_uniform(R.seed, gchain, (uint32_t)i, NUTS_TREE_BLOCK + 2u * (uint32_t)jnext) >= 0.5 ? 1 : 0;
+    T.j[c] = jnext; T.dir[c] = side; T.leaf[c] = 1; T.n_sub[c] = 0; T.alpha[c] = 0.0;
+    const double e = (side ? 1.0 : -1.0) * W.eps_cur[c];
+    const double* th_v = T.th[side];
+    const double* p_v = T.p[side];
+    const double* g_v = T.g[side];
+    for (int64_t j = 0; j < d; j++) {
+      double m = p_v[j * Cp + c];
+      m += (0.5 * g_v[j * Cp + c]) * e;                                 // HMC.jl:95
+      double p = th_v[j * Cp + c];
+      p += e * m;                                                       // HMC.jl:96
+      W.mom[j * Cp + c] = m; q[j * Cp + c] = p;
+    }
+    W.need_ll[c] = 1;
+    W.phase[c] = PH_NUTS;
+  }
+  return nev;
+}
+
+constexpr int NUTS_THREADS = 128;
+__global__ void __launch_bounds__(NUTS_THREADS) nuts_kernel(const WaveArgs W) {
+  if (!W.resume && *W.remaining == 0) return;
+  const int64_t c = (int64_t)blockIdx.x * NUTS_THREADS + threadIdx.x;
+  const int nev = (c < W.R.C) ? nuts_chain(W, c) : 0;
+  const int total = __syncthreads_count(nev);
+  if (threadIdx.x == 0 && total) atomicAdd(W.n_evals, (unsigned long long)total);
+}
+
 cudaError_t launch_transition(const WaveArgs& W, cudaStream_t st) {
+  if (W.S.kind == MCMCGPU_NUTS) {
+    nuts_kernel<<<(unsigned)((W.R.C + NUTS_THREADS - 1) / NUTS_THREADS), NUTS_THREADS, 0, st>>>(W);
+    return cudaGetLastError();
+  }
   const bool regression = (W.M.family == MCMCGPU_FAM_LINEAR || W.M.family == MCMCGPU_FAM_LOGISTIC || W.M.family == MCMCGPU_FAM_PROBIT);
   if (regression && W.S.kind != MCMCGPU_RAM && W.rb == nullptr) {
     int blocks = (int)((W.R.C + CO_CHAINS - 1) / CO_CHAINS);

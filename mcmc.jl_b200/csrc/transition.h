@@ -8,8 +8,25 @@ constexpr int PH_RWM = 1;    // q = RWM proposal has been evaluated
 constexpr int PH_MALA = 2;   // q = MALA proposal has been evaluated
 constexpr int PH_LEAP = 3;   // q = position after a leapfrog position update has been evaluated
 constexpr int PH_RAM_BEGIN = 4;  // RAM: the next proposal is made by ram_kernel (after the factor update)
+constexpr int PH_NUTS = 5;   // q = NUTS tree leaf (position after a leapfrog position update) has been evaluated
 constexpr int PH_PAUSE = 98;  // reached the step limit of this execute call; resumes at the next one
 constexpr int PH_DONE = 99;
+
+// NUTS per-chain state, chain-minor at pitch Cp (sides: 0 = backward end of the tree, 1 = forward end)
+constexpr int NUTS_MAX_DOUBLINGS = 10;
+struct NutsState {
+  double* th[2];               // [d][Cp] position of each tree end
+  double* p[2];                // [d][Cp] momentum of each tree end
+  double* g[2];                // [d][Cp] gradient of each tree end
+  double *sub_pars, *sub_grad; // [d][Cp] candidate of the subtree being built
+  double* sub_lt;              // [Cp]
+  double *ck_th, *ck_p;        // [maxdoublings][d][Cp] U-turn checkpoints: the first leaf of the open 2^r-leaf block, r = 1..j
+  double *log_u0, *alpha;      // [Cp] log slice uniform of the step; sum of min(1, exp(H0 - H)) over the current doubling
+  int32_t *j, *leaf, *leaps;   // [Cp] doubling, leaf in the subtree (1-based), leapfrogs made in the step
+  int32_t *n, *n_sub;          // [Cp] valid leaves of the tree / of the subtree
+  int32_t *dir;                // [Cp] 1: the current subtree grows forward, 0: backward
+  uint8_t* moved;              // [Cp] the step's sample is no longer the starting point
+};
 
 struct WaveArgs {
   ModelDev M;
@@ -51,9 +68,10 @@ struct WaveArgs {
   double* rb_acc;              // [d][Cp] running sum_k w_k pars_k of the current trajectory
   double* init_lt;             // [Cp] log-target at the initial point, or null
   const int64_t* chain_ids;    // [Cp] global chain id of every chain (Philox key), or null = chain_offset + position
+  NutsState nuts;              // NUTS runs only
 };
 
-cudaError_t launch_transition(const WaveArgs& W, cudaStream_t st);
+cudaError_t launch_transition(const WaveArgs& W, cudaStream_t st);   // NUTS runs: nuts_kernel
 constexpr int RAM_WAVE_MAX_D = 16;    // one thread per chain, factor in local memory; larger d: one CTA per chain (ram_big_kernel)
 constexpr int RAM_BIG_MAX_D = 128;
 cudaError_t launch_ram(const WaveArgs& W, bool init, cudaStream_t st);   // RAM.jl:50-60,73-78 for the wave engine

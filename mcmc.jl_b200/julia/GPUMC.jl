@@ -77,6 +77,8 @@ samplercfg(s::MALA)  = SamplerCfg(1, 0, s.driftStep, 0., 0., 0., 0., 0., 0, tune
 samplercfg(s::HMC)   = SamplerCfg(2, s.nLeaps, s.leapStep, 0., 0., 0., 0., 0., 0, tunercfg(s.tuner)...)
 samplercfg(s::HMCDA) = SamplerCfg(3, 0, 0., s.rate, s.len, s.shrinkage, s.t0, s.step, 0, 0, 0, 0, 0., 0.)
 samplercfg(s::RAM)   = SamplerCfg(4, 0, s.scale, s.rate, 0., 0., 0., 0., 0, 0, 0, 0, 0., 0.)
+# NUTS: nleaps = maxdoublings; rate / shrinkage / t0 / step = the dual averaging (include/mcmcgpu.h, MCMCGPU_NUTS)
+samplercfg(s::NUTS)  = SamplerCfg(5, s.maxdoublings, 0., s.rate, 0., s.shrinkage, s.t0, s.step, 0, 0, 0, 0, 0., 0.)
 
 function run_gpumc(t::MCMCTask)
   tic()

@@ -24,6 +24,9 @@ extern "C" {
 #endif
 
 #define MCMCGPU_ABI_VERSION 3   /* 2: mcmcgpu_run_info.comm_ms; 3: mcmcgpu_runner_cfg.stream_stats / stream_batchlen */
+/* The version counts changes of the structs' layouts and of existing functions.  Functions that are only added (e.g.
+ * mcmcgpu_run_set_metric) leave it as is: a binding written for version 3 keeps working, and the new symbols can be
+ * looked up by name. */
 
 /* status codes */
 #define MCMCGPU_OK 0
@@ -50,8 +53,10 @@ extern "C" {
 #define MCMCGPU_HMC 2
 #define MCMCGPU_HMCDA 3
 #define MCMCGPU_RAM 4          /* src/samplers/RAM.jl:24-36: scale, rate (robust adaptive Metropolis); d <= 8 fused, d <= 128 wave */
-/* No-U-Turn sampler: slice NUTS with dual averaging (Hoffman & Gelman 2014, Algorithms 3 and 6), identity mass matrix,
- * engine WAVE only (one leapfrog leaf per chain per wave).  It reads mcmcgpu_sampler_cfg as follows:
+/* No-U-Turn sampler: slice NUTS with dual averaging (Hoffman & Gelman 2014, Algorithms 3 and 6), with the identity or a
+ * diagonal mass matrix, fixed (mcmcgpu_run_set_metric) or adapted per chain in Stan's warm-up windows
+ * (mcmcgpu_run_set_metric_adaptation), engine WAVE only (one leapfrog leaf per chain per wave).  It reads
+ * mcmcgpu_sampler_cfg as follows:
  *   nleaps = maxdoublings (1..10: at most 2^maxdoublings - 1 leapfrogs per step);
  *   rate, shrinkage, t0, step = the dual averaging, HMCDA's rules (the target is the mean acceptance statistic of the
  *   last doubling); scale, len and max_leaps are ignored, and so is the model scale passed to the run.
@@ -178,6 +183,21 @@ int32_t mcmcgpu_run_set_state(mcmcgpu_run* run, int64_t step0, const double* lea
                               const double* dualH);
 /* current positions (d x nchains) and HMCDA / NUTS step-size state (nchains each); any pointer may be NULL */
 int32_t mcmcgpu_run_get_state(mcmcgpu_run* run, double* pars, double* leapstep, double* dual_leapstep, double* dualH);
+/* NUTS only, before the first execute: diagonal INVERSE metric, d (shared) or d x nchains (per_chain != 0); every entry
+ * finite and > 0.  Without this call the metric is the identity (the run is bit-identical to one without the call when
+ * all entries are 1).  With adaptation on it is the starting metric.  MCMCGPU_E_ARG for another sampler or a bad entry,
+ * MCMCGPU_E_STATE after the first execute. */
+int32_t mcmcgpu_run_set_metric(mcmcgpu_run* run, const double* inv_metric, int32_t per_chain);
+/* NUTS only, before the first execute: adapt every chain's diagonal metric during warm-up in Stan's windows
+ * (Stan's defaults: 75, 50, 25).  The warm-up is the W = first - 2 steps on which the step size adapts; with W < 20 the
+ * metric is not updated, and when the buffers and the window do not fit they become 15 % / 10 % of W and the rest.
+ * Each window's final samples give a Welford variance, regularised as Stan does (n / (n + 5) var + 1e-3 * 5 / (n + 5));
+ * the dual averaging then restarts at mu = log(10 eps).  Stan's step-size search at a window end is not made.  Each chain
+ * adapts alone (no pooling across chains).  Not with set_state step0 inside the warm-up (0 < step0 < first - 2).
+ * MCMCGPU_E_ARG for another sampler, negative buffers or window < 1; MCMCGPU_E_STATE after the first execute. */
+int32_t mcmcgpu_run_set_metric_adaptation(mcmcgpu_run* run, int64_t init_buffer, int64_t term_buffer, int64_t window);
+/* the current inverse metric, d x nchains (after execute / execute_steps; before, the starting metric) */
+int32_t mcmcgpu_run_get_metric(mcmcgpu_run* run, double* out_inv_metric);
 int32_t mcmcgpu_run_fetch(mcmcgpu_run* run, double* out_samples, double* out_grads, uint8_t* out_accept,
                           double* out_logtarget);
 /* Rao-Blackwellised draws (store_rb): out_rb d x S x nchains; their column means are mean_rb(chain) (mean.jl:37-41) */

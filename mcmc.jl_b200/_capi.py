@@ -57,6 +57,7 @@ EXPORTS = [
     "mcmcgpu_run_fetch", "mcmcgpu_run_fetch_rb", "mcmcgpu_run_fetch_diag", "mcmcgpu_run_stats",
     "mcmcgpu_run_destroy", "mcmcgpu_stats", "mcmcgpu_philox_draws", "mcmcgpu_run_seqmc", "mcmcgpu_run_serialtemp", "mcmcgpu_run_zv", "mcmcgpu_zv",
     "mcmcgpu_run_seqmc_models", "mcmcgpu_run_serialtemp_models",
+    "mcmcgpu_run_set_metric", "mcmcgpu_run_set_metric_adaptation", "mcmcgpu_run_get_metric",
 ]
 
 _lib = None
@@ -93,6 +94,9 @@ def lib():
         L.mcmcgpu_run_execute_steps.argtypes = [vp, C.c_int64, C.POINTER(RunInfo)]
         L.mcmcgpu_run_set_state.argtypes = [vp, C.c_int64, dp, dp, dp]
         L.mcmcgpu_run_get_state.argtypes = [vp, dp, dp, dp, dp]
+        L.mcmcgpu_run_set_metric.argtypes = [vp, dp, C.c_int32]
+        L.mcmcgpu_run_set_metric_adaptation.argtypes = [vp, C.c_int64, C.c_int64, C.c_int64]
+        L.mcmcgpu_run_get_metric.argtypes = [vp, dp]
         L.mcmcgpu_run_fetch.argtypes = [vp, dp, dp, C.POINTER(C.c_uint8), dp]
         L.mcmcgpu_run_fetch_rb.argtypes = [vp, dp]
         L.mcmcgpu_run_fetch_diag.argtypes = [vp, dp, C.POINTER(C.c_int64)]
@@ -396,6 +400,22 @@ class DeviceRun(_Owned):
         ls, du, dh = np.empty(self.C), np.empty(self.C), np.empty(self.C)
         check(lib().mcmcgpu_run_get_state(self.h, dptr(pars), dptr(ls), dptr(du), dptr(dh)))
         return dict(pars=pars, leapstep=ls, dual_leapstep=du, dualH=dh)
+
+    def set_metric(self, inv_metric):
+        """NUTS: diagonal inverse metric, (d,) for every chain or (nchains, d) per chain"""
+        m = f64(inv_metric)
+        if m.shape not in ((self.d,), (self.C, self.d)):
+            raise MCMCGPUError(E_ARG, f"inv_metric must be (d,) or (nchains, d) = {(self.C, self.d)}, got {m.shape}")
+        check(lib().mcmcgpu_run_set_metric(self.h, dptr(m), 1 if m.ndim == 2 else 0))
+
+    def set_metric_adaptation(self, init_buffer=75, term_buffer=50, window=25):
+        check(lib().mcmcgpu_run_set_metric_adaptation(self.h, int(init_buffer), int(term_buffer), int(window)))
+
+    def get_metric(self):
+        """(nchains, d) current inverse metric"""
+        out = np.empty((self.C, self.d))
+        check(lib().mcmcgpu_run_get_metric(self.h, dptr(out)))
+        return out
 
     def fetch(self, samples=True, grads=None, accept=True, logtarget=None, out=None):
         grads = self.store_grad if grads is None else grads

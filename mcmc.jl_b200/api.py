@@ -300,19 +300,40 @@ class HMCDA(_Sampler):
 
 
 class NUTS(_Sampler):
-    """No-U-Turn sampler: slice NUTS with dual averaging of the step size (Hoffman & Gelman 2014, Algorithms 3 and 6),
-    identity mass matrix.  rate is the target mean acceptance statistic, maxdoublings caps the tree at
-    2^maxdoublings - 1 leapfrogs per step, shrinkage / t0 / step are the dual averaging's gamma / t0 / kappa (HMCDA's).
-    Runs on the wave engine; the model's scale is not used."""
+    """No-U-Turn sampler: slice NUTS with dual averaging of the step size (Hoffman & Gelman 2014, Algorithms 3 and 6).
+    rate is the target mean acceptance statistic, maxdoublings caps the tree at 2^maxdoublings - 1 leapfrogs per step,
+    shrinkage / t0 / step are the dual averaging's gamma / t0 / kappa (HMCDA's).  The mass matrix is the identity unless
+    inv_metric gives a diagonal inverse metric, (d,) for every chain or (nchains, d) per chain; adapt_metric=True adapts
+    each chain's diagonal metric during warm-up in Stan's windows (init_buffer / term_buffer / window, Stan's defaults),
+    starting from inv_metric or ones.  Runs on the wave engine; the model's scale is not used."""
 
-    def __init__(self, rate=0.6, maxdoublings=10, shrinkage=0.05, t0=10.0, step=0.75):
+    def __init__(self, rate=0.6, maxdoublings=10, shrinkage=0.05, t0=10.0, step=0.75, inv_metric=None, adapt_metric=False,
+                 init_buffer=75, term_buffer=50, window=25):
         assert 0.0 < rate < 1.0, f"Target acceptance rate ({rate}) should be between 0 and 1"
         assert isinstance(maxdoublings, (int, np.integer)) and 1 <= maxdoublings <= 10, \
             f"maxdoublings parameter of NUTS sampler ({maxdoublings}) must be an integer in 1..10"
         assert shrinkage > 0.0, f"shrinkage parameter of NUTS sampler ({shrinkage}) must be positive"
         assert t0 >= 0, f"t0 parameter of NUTS sampler ({t0}) must be non-negative"
+        if inv_metric is not None:
+            inv_metric = np.array(inv_metric, dtype=np.float64)
+            assert inv_metric.ndim in (1, 2) and inv_metric.size > 0, \
+                f"inv_metric of NUTS sampler must be (d,) or (nchains, d), got shape {inv_metric.shape}"
+            assert np.all(np.isfinite(inv_metric)) and np.all(inv_metric > 0), "inv_metric of NUTS sampler must be positive and finite"
+        for name, v, lo in (("init_buffer", init_buffer, 0), ("term_buffer", term_buffer, 0), ("window", window, 1)):
+            assert isinstance(v, (int, np.integer)) and v >= lo, f"{name} of NUTS sampler ({v}) must be an integer >= {lo}"
         self.rate, self.maxdoublings, self.shrinkage, self.t0, self.step = rate, int(maxdoublings), shrinkage, t0, step
+        self.inv_metric, self.adapt_metric = inv_metric, bool(adapt_metric)
+        self.init_buffer, self.term_buffer, self.window = int(init_buffer), int(term_buffer), int(window)
         self.tuner = None
+
+    def _set_metric(self, drun, offset, nchains):
+        """the metric calls of a run of chains offset .. offset + drun.C - 1 of nchains (none with the defaults)"""
+        if self.inv_metric is not None:
+            assert self.inv_metric.ndim == 1 or self.inv_metric.shape[0] == nchains, \
+                f"inv_metric of NUTS sampler has {self.inv_metric.shape[0]} rows for {nchains} chains"
+            drun.set_metric(self.inv_metric if self.inv_metric.ndim == 1 else self.inv_metric[offset:offset + drun.C])
+        if self.adapt_metric:
+            drun.set_metric_adaptation(self.init_buffer, self.term_buffer, self.window)
 
     def _cfg(self):
         return capi.sampler_cfg("NUTS", nleaps=self.maxdoublings, rate=self.rate, shrinkage=self.shrinkage, t0=self.t0,
@@ -494,10 +515,13 @@ class MCMCChainBatch:
     def __getitem__(self, i):
         a = self.arrays()
         diags = {"step": np.array(list(self.range)), "accept": a["accept"][i].astype(bool)}
-        if isinstance(self.task.sampler, NUTS):
+        s = self.task.sampler
+        if isinstance(s, NUTS):
             eps, leaps = self.diag()
             diags["epsilon"] = eps[i]
             diags["ndoublings"] = np.floor(np.log2(leaps[i])).astype(np.int64) + 1    # the tree of 2^(n-1) .. 2^n - 1 leapfrogs
+            if s.inv_metric is not None or s.adapt_metric:
+                diags["inv_metric"] = self.inv_metric()[i]
         g = a.get("grads")
         return MCMCChain(self.range, a["samples"][i], None if g is None else g[i], diags, self.task, self.runTime,
                          _colnames(self.task.model))
@@ -510,6 +534,12 @@ class MCMCChainBatch:
         if getattr(self, "_diag", None) is None:
             self._diag = self._run.fetch_diag()
         return self._diag
+
+    def inv_metric(self):
+        """(C, d) diagonal inverse metric of every chain at the end of the run (NUTS; ones for the identity)"""
+        if getattr(self, "_minv", None) is None:
+            self._minv = self._run.get_metric()
+        return self._minv
 
     def stats(self, vtype="imse", **kw):
         return self._run.stats(vtype, kw.get("maxlag", -1), kw.get("batchlen", 100))
@@ -592,7 +622,12 @@ def _run_task(t, init=None, normals=None, uniforms=None, shard_over_ranks=False)
                           store_grad=bool(r.store_gradients) and not stream, store_logtarget=not stream,
                           engine="fused" if stream else r.engine, store_rb=bool(getattr(s, "storeLeaps", False)), stream_stats=stream)
     try:
+        if isinstance(s, NUTS):
+            s._set_metric(drun, offset, r.nchains)
         info = drun.execute()
+    except AssertionError:
+        drun.close()
+        raise
     except MCMCGPUError as e:
         drun.close()
         if e.code == capi.E_SUPPORT:

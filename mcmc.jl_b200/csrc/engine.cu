@@ -1,6 +1,7 @@
 // engine.cu -- host side of libmcmcgpu.so: the C ABI of include/mcmcgpu.h (contexts, models, runs).
 // No CPU fallback exists: every compute entry point needs a CUDA device and fails with
 // MCMCGPU_E_CUDA otherwise.
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -107,6 +108,7 @@ struct mcmcgpu_run {
   int64_t *istep = nullptr, *kept = nullptr, *tn_nleaps = nullptr, *tn_acc = nullptr, *tn_prop = nullptr;
   uint8_t *need_ll = nullptr, *k1_done = nullptr;
   NutsState nuts{};          // NUTS runs only
+  bool adapt_metric = false; // NUTS: mcmcgpu_run_set_metric_adaptation was called
   int nsplit = 1;
   std::vector<void*> owned, owned_big;
   template <typename T>
@@ -875,6 +877,9 @@ int32_t mcmcgpu_run_execute_steps(mcmcgpu_run* R, int64_t nsteps, mcmcgpu_run_in
   return execute_impl(R, nsteps, info);
 }
 
+// metric adaptation needs the whole warm-up: a run may start at step0 = 0 or after the warm-up
+static bool step0_in_warmup(const mcmcgpu_run* R, int64_t step0) { return step0 > 0 && step0 < R->r.first - 2; }
+
 static int upload_chain_vec(mcmcgpu_run* R, double* dst, const double* src) {
   return cudaMemcpyAsync(dst, src, sizeof(double) * (size_t)R->C, cudaMemcpyHostToDevice, R->m->ctx->stream) == cudaSuccess
              ? MCMCGPU_OK : fail(MCMCGPU_E_CUDA, "CUDA: state upload failed");
@@ -887,6 +892,7 @@ int32_t mcmcgpu_run_set_state(mcmcgpu_run* R, int64_t step0, const double* leaps
   if (R->engine != MCMCGPU_ENGINE_WAVE) return fail(MCMCGPU_E_STATE, "mcmcgpu_run_set_state needs engine WAVE");
   if (step0 < 0 || step0 >= R->r.last) return fail(MCMCGPU_E_ARG, "step0 must be in [0, last)");
   if (R->r.first <= step0) return fail(MCMCGPU_E_ARG, "the kept range must start after step0");
+  if (R->adapt_metric && step0_in_warmup(R, step0)) return fail(MCMCGPU_E_ARG, "metric adaptation cannot start inside the warm-up (set_state step0)");
   CU(use_ctx(R->m->ctx));
   R->step0 = step0;
   if (leapstep || dual_leapstep || dualH) {
@@ -899,6 +905,105 @@ int32_t mcmcgpu_run_set_state(mcmcgpu_run* R, int64_t step0, const double* leaps
     CU(cudaStreamSynchronize(R->m->ctx->stream));
     R->restore_da = true;
   }
+  return MCMCGPU_OK;
+}
+
+// Stan's adaptation windows (windowed_adaptation.hpp) over the W = first - 2 warm-up steps on which the dual averaging
+// adapts; the window counter of step i is k = i - 1.  Returns the window-end steps and the steps lo..hi whose samples
+// enter the variance estimate (none when W < 20).
+static std::vector<int64_t> metric_windows(int64_t W, int64_t init, int64_t term, int64_t window, int64_t* lo, int64_t* hi) {
+  std::vector<int64_t> ends;
+  *lo = 1; *hi = 0;
+  if (W < 20) return ends;
+  if (init > W || term > W || window > W || init + window + term > W) {
+    init = (int64_t)(0.15 * (double)W); term = (int64_t)(0.1 * (double)W); window = W - (init + term);
+  }
+  const int64_t last = W - term - 1;       // the last window ends here
+  int64_t size = window, next = init + window - 1;
+  for (;;) {                               // at the end of the window that ends at k = next:
+    ends.push_back(next + 1);
+    if (next == last) break;
+    size *= 2;
+    next += size;
+    if (next != last && next + 2 * size >= W - term) next = last;
+  }
+  *lo = init + 1; *hi = W - term;
+  return ends;
+}
+
+// the starting metric of every chain from a host array of C x d (chain-major), allocated on first use
+static int upload_metric(mcmcgpu_run* R, const double* host) {
+  cudaStream_t st = R->m->ctx->stream;
+  if (!R->nuts.minv) CU(R->alloc(&R->nuts.minv, (size_t)(R->d * R->Cp)));
+  double* tmp = nullptr;
+  DevBufs staging;
+  CU(staging.up(&tmp, host, (size_t)(R->C * R->d), st));
+  CU(transpose_to_chain_minor(tmp, R->nuts.minv, R->C, R->d, R->Cp, st));
+  CU(cudaStreamSynchronize(st));
+  return MCMCGPU_OK;
+}
+
+int32_t mcmcgpu_run_set_metric(mcmcgpu_run* R, const double* inv_metric, int32_t per_chain) {
+  if (!R || !inv_metric) return fail(MCMCGPU_E_ARG, "NULL argument");
+  if (R->s.kind != MCMCGPU_NUTS) return fail(MCMCGPU_E_ARG, "a metric applies to NUTS");
+  if (R->started) return fail(MCMCGPU_E_STATE, "the metric must be set before the first execute");
+  const int64_t C = R->C, d = R->d, n = per_chain ? C * d : d;
+  for (int64_t k = 0; k < n; k++)
+    if (!(std::isfinite(inv_metric[k]) && inv_metric[k] > 0)) return fail(MCMCGPU_E_ARG, "every inverse metric entry must be finite and > 0");
+  CU(use_ctx(R->m->ctx));
+  if (per_chain) return upload_metric(R, inv_metric);
+  std::vector<double> all((size_t)(C * d));
+  for (int64_t c = 0; c < C; c++) std::copy(inv_metric, inv_metric + d, all.begin() + c * d);
+  return upload_metric(R, all.data());
+}
+
+int32_t mcmcgpu_run_set_metric_adaptation(mcmcgpu_run* R, int64_t init_buffer, int64_t term_buffer, int64_t window) {
+  if (!R) return fail(MCMCGPU_E_ARG, "run is NULL");
+  if (R->s.kind != MCMCGPU_NUTS) return fail(MCMCGPU_E_ARG, "metric adaptation applies to NUTS");
+  if (R->started) return fail(MCMCGPU_E_STATE, "metric adaptation must be set before the first execute");
+  if (init_buffer < 0 || term_buffer < 0 || window < 1) return fail(MCMCGPU_E_ARG, "adaptation buffers must be >= 0 and the window >= 1");
+  if (step0_in_warmup(R, R->step0)) return fail(MCMCGPU_E_ARG, "metric adaptation cannot start inside the warm-up (set_state step0)");
+  CU(use_ctx(R->m->ctx));
+  NutsState& T = R->nuts;
+  if (!T.minv) {
+    std::vector<double> ones((size_t)(R->C * R->d), 1.0);
+    int rc = upload_metric(R, ones.data());
+    if (rc) return rc;
+  }
+  int64_t lo, hi;
+  const std::vector<int64_t> ends = metric_windows(R->r.first - 2, init_buffer, term_buffer, window, &lo, &hi);
+  if (!T.wf_mean) {
+    CU(R->alloc(&T.wf_mean, (size_t)(R->d * R->Cp)));
+    CU(R->alloc(&T.wf_m2, (size_t)(R->d * R->Cp)));
+    CU(R->alloc(&T.wf_n, (size_t)R->Cp));
+    CU(R->alloc(&T.da_eps0, (size_t)R->Cp));
+    CU(R->alloc(&T.da_i0, (size_t)R->Cp));
+  }
+  int64_t* win_end = nullptr;
+  CU(R->alloc(&win_end, ends.size()));
+  T.win_end = win_end;
+  if (!ends.empty()) CU(cudaMemcpyAsync(win_end, ends.data(), sizeof(int64_t) * ends.size(), cudaMemcpyHostToDevice, R->m->ctx->stream));
+  CU(cudaStreamSynchronize(R->m->ctx->stream));
+  T.n_win = (int32_t)ends.size(); T.win_lo = lo; T.win_hi = hi;
+  R->adapt_metric = true;
+  return MCMCGPU_OK;
+}
+
+int32_t mcmcgpu_run_get_metric(mcmcgpu_run* R, double* out_inv_metric) {
+  if (!R || !out_inv_metric) return fail(MCMCGPU_E_ARG, "NULL argument");
+  if (R->s.kind != MCMCGPU_NUTS) return fail(MCMCGPU_E_ARG, "a metric applies to NUTS");
+  if (!R->nuts.minv) {
+    std::fill(out_inv_metric, out_inv_metric + R->C * R->d, 1.0);
+    return MCMCGPU_OK;
+  }
+  CU(use_ctx(R->m->ctx));
+  cudaStream_t st = R->m->ctx->stream;
+  double* tmp = nullptr;
+  DevBufs bufs;
+  CU(bufs.get(&tmp, (size_t)(R->C * R->d), st, false));
+  CU(transpose_to_chain_major(R->nuts.minv, tmp, 0, R->C, R->d, R->Cp, st));
+  CU(cudaMemcpyAsync(out_inv_metric, tmp, sizeof(double) * (size_t)(R->C * R->d), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
   return MCMCGPU_OK;
 }
 

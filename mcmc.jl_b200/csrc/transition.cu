@@ -114,14 +114,18 @@ __device__ __forceinline__ void store_kept(const WaveArgs& W, const int64_t c, i
 }
 
 // The dual-averaging update of step i < burnin (HMCDA.jl:133-138), shared by HMCDA (pacc = its acceptance probability)
-// and NUTS (pacc = the mean acceptance statistic of the step's last doubling).
+// and NUTS (pacc = the mean acceptance statistic of the step's last doubling).  The averaging counts steps from i0 and
+// shrinks towards mu = log(ten_eps0): HMCDA passes 10 * leapStep0 (leapStep0 = 1) and i0 = 0; NUTS with metric adaptation
+// restarts it at every window end (i0 = that step, ten_eps0 = 10 eps).  The log is taken here, where HMCDA always took it,
+// so that the HMCDA kernels compile to the same instructions.
 struct DaStep { double leapstep, dual, dualH; };
-__device__ __forceinline__ DaStep da_adapt(const SamplerDev& S, int64_t i, double pacc, double dual, double dualH) {
-  const double fi = (double)i;
+__device__ __forceinline__ DaStep da_adapt(const SamplerDev& S, int64_t i, double pacc, double dual, double dualH,
+                                           double ten_eps0, int64_t i0) {
+  const double fi = (double)(i - i0);
   double eta = 1.0 / (fi + S.t0);
   DaStep r;
   r.dualH = (1.0 - eta) * dualH + eta * (S.rate - pacc);
-  r.leapstep = exp(log(10.0 * 1.0) - sqrt(fi) * r.dualH / S.shrinkage);   // mu = log(10*leapStep0), leapStep0 = 1
+  r.leapstep = exp(log(ten_eps0) - sqrt(fi) * r.dualH / S.shrinkage);
   eta = pow(fi, -S.step);
   r.dual = exp((1.0 - eta) * log(dual) + eta * log(r.leapstep));
   return r;
@@ -290,7 +294,7 @@ __device__ int transition_chain(const WaveArgs& W, const int64_t c, const bool i
     store(i, true, acc, eps, nl_cur);
     if (kind == MCMCGPU_HMCDA) {
       if (i < burnin) {                                               // HMCDA.jl:133-138
-        const DaStep a = da_adapt(S, i, pacc, W.da_dual[c], W.da_dualH[c]);
+        const DaStep a = da_adapt(S, i, pacc, W.da_dual[c], W.da_dualH[c], 10.0 * 1.0, 0);
         W.da_dual[c] = a.dual; W.da_dualH[c] = a.dualH; W.da_leapstep[c] = a.leapstep;
       } else {
         W.da_leapstep[c] = W.da_dual[c];                              // :140
@@ -653,7 +657,7 @@ __global__ void __launch_bounds__(CO_CHAINS * CO_GROUPS, 2) transition_coop_kern
         stored = true; st_eps = eps_cur; st_nl = nlc;
         if (kind == MCMCGPU_HMCDA) {
           if (i < burnin) {                                               // HMCDA.jl:133-138
-            const DaStep a = da_adapt(S, i, pacc, da_dual_ld, da_dualH_ld);
+            const DaStep a = da_adapt(S, i, pacc, da_dual_ld, da_dualH_ld, 10.0 * 1.0, 0);
             W.da_dual[c] = a.dual; W.da_dualH[c] = a.dualH; W.da_leapstep[c] = a.leapstep; da_ls_ld = a.leapstep;
           } else {
             W.da_leapstep[c] = da_dual_ld; da_ls_ld = da_dual_ld;         // :140
@@ -810,19 +814,66 @@ __global__ void __launch_bounds__(CO_CHAINS * CO_GROUPS, 2) transition_coop_kern
 // recursion makes.  Draws of step i: momentum from the normal blocks, slice uniform u0 from block 0xFFFFFFFF, direction
 // of doubling j from NUTS_TREE_BLOCK + 2j, its merge from NUTS_TREE_BLOCK + 2j + 1, candidate choice of the step's leaf
 // k (0-based) from NUTS_LEAF_BLOCK + k.  One thread per chain; every array is chain-minor, so a warp's accesses coalesce.
+//
+// MET: a diagonal inverse metric minv = M^-1 (NutsState::minv).  It enters as p = z / sqrt(minv), K = 0.5 sum (minv p) p,
+// theta += e (minv m) and the U-turn dots delta . (minv p); with MET = false every one of these is the identity's operation
+// and minv is never loaded.  (z / 1, 1 * p and 1 * m are exact, so an all-ones metric gives the identity's bits.)
 
-// continue (true) unless a U-turn: delta = v (theta_m - theta_s), delta . p_s >= 0 and delta . p_m >= 0, summed in j order
+// minv_j * x, or x itself for the identity metric
+template <bool MET>
+__device__ __forceinline__ double nuts_mv(const double* minv, int64_t jc, double x) {
+  if constexpr (MET) return minv[jc] * x;
+  else return x;
+}
+
+// continue (true) unless a U-turn: delta = v (theta_m - theta_s), delta . (minv p_s) >= 0 and delta . (minv p_m) >= 0,
+// summed in j order
+template <bool MET>
 __device__ __forceinline__ bool nuts_no_uturn(const double* th_m, const double* p_m, const double* th_s, const double* p_s, double v,
-                                              int64_t d, int64_t Cp, int64_t c) {
+                                              const double* minv, int64_t d, int64_t Cp, int64_t c) {
   double ds = 0.0, dm = 0.0;
   for (int64_t j = 0; j < d; j++) {
     const double delta = v * (th_m[j * Cp + c] - th_s[j * Cp + c]);
-    ds += delta * p_s[j * Cp + c];
-    dm += delta * p_m[j * Cp + c];
+    ds += delta * nuts_mv<MET>(minv, j * Cp + c, p_s[j * Cp + c]);
+    dm += delta * nuts_mv<MET>(minv, j * Cp + c, p_m[j * Cp + c]);
   }
   return ds >= 0.0 && dm >= 0.0;
 }
 
+// Metric adaptation after the dual-averaging update of warm-up step i (Stan's var_adaptation::learn_variance and the
+// step-size restart of adapt_diag_e_nuts::transition): the step's final sample joins the window's Welford sums; at a
+// window end the variance estimate, regularised towards 1e-3, becomes the metric, the sums restart and the dual averaging
+// restarts at mu = log(10 eps) from step i (eps: the step size the update just made, which the next step uses).
+__device__ void nuts_adapt_metric(const WaveArgs& W, const int64_t c, int64_t i, double eps) {
+  const NutsState& T = W.nuts;
+  const int64_t d = W.M.d, Cp = W.R.Cp;
+  if (i >= T.win_lo && i <= T.win_hi) {
+    const double n = (double)(T.wf_n[c] + 1);
+    T.wf_n[c] += 1;
+    for (int64_t j = 0; j < d; j++) {
+      const double x = W.cur_pars[j * Cp + c];
+      double mean = T.wf_mean[j * Cp + c];
+      const double delta = x - mean;
+      mean += delta / n;
+      T.wf_mean[j * Cp + c] = mean;
+      T.wf_m2[j * Cp + c] += delta * (x - mean);
+    }
+  }
+  bool end = false;
+  for (int k = 0; k < T.n_win; k++) end |= T.win_end[k] == i;
+  if (!end) return;
+  const double n = (double)T.wf_n[c];
+  for (int64_t j = 0; j < d; j++) {
+    const double var = n > 1.0 ? T.wf_m2[j * Cp + c] / (n - 1.0) : T.minv[j * Cp + c];   // one draw: the metric stays
+    T.minv[j * Cp + c] = (n / (n + 5.0)) * var + 1e-3 * (5.0 / (n + 5.0));
+    T.wf_mean[j * Cp + c] = 0.0; T.wf_m2[j * Cp + c] = 0.0;
+  }
+  T.wf_n[c] = 0;
+  T.da_eps0[c] = eps; T.da_i0[c] = i;
+  W.da_dual[c] = 1.0; W.da_dualH[c] = 0.0;
+}
+
+template <bool MET>
 __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
   const RunnerDev& R = W.R;
   const SamplerDev& S = W.S;
@@ -862,6 +913,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       W.cur_grad[j * Cp + c] = fin_grad(F, M, q, part, ns, Cp, c, j);
     }
     if (!W.restore_da) { W.da_leapstep[c] = 1.0; W.da_dual[c] = 1.0; W.da_dualH[c] = 0.0; }   // eps0 = 1, as HMCDA
+    if constexpr (MET) if (T.win_end) { T.da_eps0[c] = 1.0; T.da_i0[c] = 0; }
     i = W.step0 + 1;
     begin = true;
   } else {   // PH_NUTS: leaf `leaf` of the subtree of doubling jd has been evaluated at q
@@ -877,7 +929,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       const double gj = fin_grad(F, M, q, part, ns, Cp, c, j);
       double m = W.mom[j * Cp + c];
       m += (0.5 * gj) * e;
-      mm += m * m;
+      mm += nuts_mv<MET>(T.minv, j * Cp + c, m) * m;
       th_v[j * Cp + c] = q[j * Cp + c]; p_v[j * Cp + c] = m; g_v[j * Cp + c] = gj;
     }
     const double H = -F.lt + 0.5 * mm;                                  // update! HMC.jl:91
@@ -898,7 +950,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
     }
     const int64_t slot = d * Cp;
     for (int r = 1; s && r <= jd && (leaf & ((1 << r) - 1)) == 0; r++)        // U-turn checks of the blocks this leaf closes
-      s = nuts_no_uturn(th_v, p_v, T.ck_th + (r - 1) * slot, T.ck_p + (r - 1) * slot, v, d, Cp, c);
+      s = nuts_no_uturn<MET>(th_v, p_v, T.ck_th + (r - 1) * slot, T.ck_p + (r - 1) * slot, v, T.minv, d, Cp, c);
     bool open = false;
     if (s && leaf < (1 << jd)) {                                        // next leaf of this subtree
       for (int r = 1; r <= jd && ((leaf - 1) & ((1 << r) - 1)) == 0; r++)     // checkpoints of the blocks this leaf opens
@@ -910,7 +962,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
         double m = p_v[j * Cp + c];
         m += (0.5 * g_v[j * Cp + c]) * e;
         double p = th_v[j * Cp + c];
-        p += e * m;
+        p += e * nuts_mv<MET>(T.minv, j * Cp + c, m);
         W.mom[j * Cp + c] = m; q[j * Cp + c] = p;
       }
       T.leaf[c] = leaf + 1;
@@ -923,7 +975,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
         T.moved[c] = 1;
       }
       T.n[c] = n + nsub;
-      open = jd + 1 < S.nleaps && nuts_no_uturn(T.th[1], T.p[1], T.th[0], T.p[0], 1.0, d, Cp, c);
+      open = jd + 1 < S.nleaps && nuts_no_uturn<MET>(T.th[1], T.p[1], T.th[0], T.p[0], 1.0, T.minv, d, Cp, c);
     }
     if (open) {
       doubling = true; jnext = jd + 1;
@@ -931,8 +983,12 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       const double pacc = alpha / (double)leaf;                         // alpha / n_alpha of the last doubling
       store_kept(W, c, i, true, T.moved[c] != 0, W.eps_cur[c], k + 1);
       if (i < burnin) {
-        const DaStep a = da_adapt(S, i, pacc, W.da_dual[c], W.da_dualH[c]);
+        double eps0 = 1.0;
+        int64_t i0 = 0;
+        if constexpr (MET) if (T.win_end) { eps0 = T.da_eps0[c]; i0 = T.da_i0[c]; }
+        const DaStep a = da_adapt(S, i, pacc, W.da_dual[c], W.da_dualH[c], 10.0 * eps0, i0);
         W.da_dual[c] = a.dual; W.da_dualH[c] = a.dualH; W.da_leapstep[c] = a.leapstep;
+        if constexpr (MET) if (T.win_end) nuts_adapt_metric(W, c, i, a.leapstep);
       } else {
         W.da_leapstep[c] = W.da_dual[c];
       }
@@ -962,8 +1018,9 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       for (int t = 0; t < 2; t++) {
         const int64_t j = jb + t;
         if (j >= d) break;
-        const double z = t ? z1 : z0;
-        mm += z * z;
+        double z = t ? z1 : z0;
+        if constexpr (MET) z = z / sqrt(T.minv[j * Cp + c]);                  // p = z / sqrt(minv)
+        mm += nuts_mv<MET>(T.minv, j * Cp + c, z) * z;
         const double pj = W.cur_pars[j * Cp + c], gj = W.cur_grad[j * Cp + c];
         T.th[0][j * Cp + c] = pj; T.th[1][j * Cp + c] = pj;
         T.p[0][j * Cp + c] = z; T.p[1][j * Cp + c] = z;
@@ -987,7 +1044,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       double m = p_v[j * Cp + c];
       m += (0.5 * g_v[j * Cp + c]) * e;                                 // HMC.jl:95
       double p = th_v[j * Cp + c];
-      p += e * m;                                                       // HMC.jl:96
+      p += e * nuts_mv<MET>(T.minv, j * Cp + c, m);                     // HMC.jl:96
       W.mom[j * Cp + c] = m; q[j * Cp + c] = p;
     }
     W.need_ll[c] = 1;
@@ -997,17 +1054,20 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
 }
 
 constexpr int NUTS_THREADS = 128;
+template <bool MET>
 __global__ void __launch_bounds__(NUTS_THREADS) nuts_kernel(const WaveArgs W) {
   if (!W.resume && *W.remaining == 0) return;
   const int64_t c = (int64_t)blockIdx.x * NUTS_THREADS + threadIdx.x;
-  const int nev = (c < W.R.C) ? nuts_chain(W, c) : 0;
+  const int nev = (c < W.R.C) ? nuts_chain<MET>(W, c) : 0;
   const int total = __syncthreads_count(nev);
   if (threadIdx.x == 0 && total) atomicAdd(W.n_evals, (unsigned long long)total);
 }
 
 cudaError_t launch_transition(const WaveArgs& W, cudaStream_t st) {
   if (W.S.kind == MCMCGPU_NUTS) {
-    nuts_kernel<<<(unsigned)((W.R.C + NUTS_THREADS - 1) / NUTS_THREADS), NUTS_THREADS, 0, st>>>(W);
+    const unsigned blocks = (unsigned)((W.R.C + NUTS_THREADS - 1) / NUTS_THREADS);
+    if (W.nuts.minv) nuts_kernel<true><<<blocks, NUTS_THREADS, 0, st>>>(W);
+    else nuts_kernel<false><<<blocks, NUTS_THREADS, 0, st>>>(W);
     return cudaGetLastError();
   }
   const bool regression = (W.M.family == MCMCGPU_FAM_LINEAR || W.M.family == MCMCGPU_FAM_LOGISTIC || W.M.family == MCMCGPU_FAM_PROBIT);

@@ -26,6 +26,18 @@ struct NutsState {
   int32_t *n, *n_sub;          // [Cp] valid leaves of the tree / of the subtree
   int32_t *dir;                // [Cp] 1: the current subtree grows forward, 0: backward
   uint8_t* moved;              // [Cp] the step's sample is no longer the starting point
+  // diagonal inverse metric M^-1 (mcmcgpu_run_set_metric / _set_metric_adaptation).  Null: the identity, and nuts_kernel's
+  // identity instantiation, which loads nothing
+  double* minv;                // [d][Cp]
+  // metric adaptation in Stan's windows (null win_end: off).  Steps win_lo..win_hi add their final sample to the Welford
+  // sums; at each of the n_win window-end steps the metric is re-estimated and the dual averaging restarts
+  double *wf_mean, *wf_m2;     // [d][Cp] Welford mean and sum of squared deviations of the current window
+  int64_t* wf_n;               // [Cp] samples in the current window
+  double* da_eps0;             // [Cp] step size of the last restart: the dual averaging's mu = log(10 da_eps0)
+  int64_t* da_i0;              // [Cp] step of the last restart (the dual averaging counts steps from it)
+  const int64_t* win_end;      // [n_win] ascending
+  int64_t win_lo, win_hi;
+  int32_t n_win;
 };
 
 struct WaveArgs {

@@ -80,6 +80,26 @@ samplercfg(s::RAM)   = SamplerCfg(4, 0, s.scale, s.rate, 0., 0., 0., 0., 0, 0, 0
 # NUTS: nleaps = maxdoublings; rate / shrinkage / t0 / step = the dual averaging (include/mcmcgpu.h, MCMCGPU_NUTS)
 samplercfg(s::NUTS)  = SamplerCfg(5, s.maxdoublings, 0., s.rate, 0., s.shrinkage, s.t0, s.step, 0, 0, 0, 0, 0., 0.)
 
+# NUTS's diagonal metric on a run handle (mcmcgpu_run_create), before its first execute.  The NUTS type carries
+#   invmetric::Union(Nothing, Array{Float64})   # d, or d x nchains; nothing = the identity
+#   adaptmetric::Bool; initbuffer::Int; termbuffer::Int; window::Int   # Stan's windows, defaults 75 / 50 / 25
+function nuts_metric!(run::Ptr{Void}, s::NUTS)
+  if s.invmetric != nothing
+    check(ccall((:mcmcgpu_run_set_metric, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}, Int32),
+                run, s.invmetric, ndims(s.invmetric) == 2 ? 1 : 0))
+  end
+  if s.adaptmetric
+    check(ccall((:mcmcgpu_run_set_metric_adaptation, libmcmcgpu), Int32, (Ptr{Void}, Int64, Int64, Int64),
+                run, s.initbuffer, s.termbuffer, s.window))
+  end
+end
+# the d x nchains inverse metric of a run (after execute: the adapted one)
+function nuts_metric(run::Ptr{Void}, d::Int, nchains::Int)
+  out = Array(Float64, d, nchains)
+  check(ccall((:mcmcgpu_run_get_metric, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}), run, out))
+  out
+end
+
 function run_gpumc(t::MCMCTask)
   tic()
   m, r = t.model, t.runner

@@ -53,9 +53,9 @@ extern "C" {
 #define MCMCGPU_HMC 2
 #define MCMCGPU_HMCDA 3
 #define MCMCGPU_RAM 4          /* src/samplers/RAM.jl:24-36: scale, rate (robust adaptive Metropolis); d <= 8 fused, d <= 128 wave */
-/* No-U-Turn sampler: slice NUTS with dual averaging (Hoffman & Gelman 2014, Algorithms 3 and 6), with the identity or a
- * diagonal mass matrix, fixed (mcmcgpu_run_set_metric) or adapted per chain in Stan's warm-up windows
- * (mcmcgpu_run_set_metric_adaptation), engine WAVE only (one leapfrog leaf per chain per wave).  It reads
+/* No-U-Turn sampler: slice NUTS with dual averaging (Hoffman & Gelman 2014, Algorithms 3 and 6), with the identity, a
+ * diagonal or a dense mass matrix, fixed (mcmcgpu_run_set_metric / _set_dense_metric) or adapted per chain in Stan's
+ * warm-up windows (mcmcgpu_run_set_metric_adaptation), engine WAVE only (one leapfrog leaf per chain per wave).  It reads
  * mcmcgpu_sampler_cfg as follows:
  *   nleaps = maxdoublings (1..10: at most 2^maxdoublings - 1 leapfrogs per step);
  *   rate, shrinkage, t0, step = the dual averaging, HMCDA's rules (the target is the mean acceptance statistic of the
@@ -196,8 +196,24 @@ int32_t mcmcgpu_run_set_metric(mcmcgpu_run* run, const double* inv_metric, int32
  * adapts alone (no pooling across chains).  Not with set_state step0 inside the warm-up (0 < step0 < first - 2).
  * MCMCGPU_E_ARG for another sampler, negative buffers or window < 1; MCMCGPU_E_STATE after the first execute. */
 int32_t mcmcgpu_run_set_metric_adaptation(mcmcgpu_run* run, int64_t init_buffer, int64_t term_buffer, int64_t window);
-/* the current inverse metric, d x nchains (after execute / execute_steps; before, the starting metric) */
+/* the current inverse metric, d x nchains (after execute / execute_steps; before, the starting metric).  MCMCGPU_E_ARG on
+ * a run with a dense metric. */
 int32_t mcmcgpu_run_get_metric(mcmcgpu_run* run, double* out_inv_metric);
+/* NUTS only, before the first execute: a dense INVERSE metric M^-1 (Stan's dense_e), d x d shared by every chain, or
+ * d x d x nchains (per_chain != 0), column-major: element (i, j) of chain c at (c*d + j)*d + i.  NULL: the identity.  Every
+ * matrix must be finite, exactly symmetric and positive definite (the Cholesky factorisation the kernel uses succeeds).
+ * Arithmetic (DESIGN.md, NUTS): p = L^-T z with A = L L^T; K = 0.5 m . (A m); theta += e (A m); U-turn dots delta . (A p).
+ * A diagonal A gives the bits of mcmcgpu_run_set_metric with its diagonal, the identity those of a run without a metric.
+ * A following mcmcgpu_run_set_metric_adaptation adapts the dense metric per chain in Stan's windows from a Welford
+ * covariance: A = (n / (n + 5)) cov + 1e-3 (5 / (n + 5)) I; a chain whose new A fails the Cholesky keeps its previous A.
+ * MCMCGPU_E_ARG for another sampler, a bad matrix, a run that has a diagonal metric or already adapts one;
+ * MCMCGPU_E_STATE after the first execute.  Memory: A and L (d*d doubles each) per chain, or once when shared and fixed;
+ * with adaptation also the d*d Welford sums per chain. */
+int32_t mcmcgpu_run_set_dense_metric(mcmcgpu_run* run, const double* inv_metric, int32_t per_chain);
+/* the current dense inverse metric, d x d x nchains column-major as above (before execute: the starting one).  An adapted
+ * metric is Stan's unsymmetrised covariance estimate, so it need not be exactly symmetric.  MCMCGPU_E_ARG on a run
+ * without a dense metric. */
+int32_t mcmcgpu_run_get_dense_metric(mcmcgpu_run* run, double* out);
 int32_t mcmcgpu_run_fetch(mcmcgpu_run* run, double* out_samples, double* out_grads, uint8_t* out_accept,
                           double* out_logtarget);
 /* Rao-Blackwellised draws (store_rb): out_rb d x S x nchains; their column means are mean_rb(chain) (mean.jl:37-41) */

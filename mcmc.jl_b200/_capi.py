@@ -58,6 +58,7 @@ EXPORTS = [
     "mcmcgpu_run_destroy", "mcmcgpu_stats", "mcmcgpu_philox_draws", "mcmcgpu_run_seqmc", "mcmcgpu_run_serialtemp", "mcmcgpu_run_zv", "mcmcgpu_zv",
     "mcmcgpu_run_seqmc_models", "mcmcgpu_run_serialtemp_models",
     "mcmcgpu_run_set_metric", "mcmcgpu_run_set_metric_adaptation", "mcmcgpu_run_get_metric",
+    "mcmcgpu_run_set_dense_metric", "mcmcgpu_run_get_dense_metric",
 ]
 
 _lib = None
@@ -97,6 +98,8 @@ def lib():
         L.mcmcgpu_run_set_metric.argtypes = [vp, dp, C.c_int32]
         L.mcmcgpu_run_set_metric_adaptation.argtypes = [vp, C.c_int64, C.c_int64, C.c_int64]
         L.mcmcgpu_run_get_metric.argtypes = [vp, dp]
+        L.mcmcgpu_run_set_dense_metric.argtypes = [vp, dp, C.c_int32]
+        L.mcmcgpu_run_get_dense_metric.argtypes = [vp, dp]
         L.mcmcgpu_run_fetch.argtypes = [vp, dp, dp, C.POINTER(C.c_uint8), dp]
         L.mcmcgpu_run_fetch_rb.argtypes = [vp, dp]
         L.mcmcgpu_run_fetch_diag.argtypes = [vp, dp, C.POINTER(C.c_int64)]
@@ -416,6 +419,24 @@ class DeviceRun(_Owned):
         out = np.empty((self.C, self.d))
         check(lib().mcmcgpu_run_get_metric(self.h, dptr(out)))
         return out
+
+    def set_dense_metric(self, inv_metric=None):
+        """NUTS: dense inverse metric, (d, d) for every chain or (nchains, d, d) per chain; None = the identity"""
+        if inv_metric is None:
+            check(lib().mcmcgpu_run_set_dense_metric(self.h, None, 0))
+            return
+        m = f64(inv_metric)
+        d = self.d
+        if m.shape not in ((d, d), (self.C, d, d)):
+            raise MCMCGPUError(E_ARG, f"inv_metric must be (d, d) or (nchains, d, d) = {(self.C, d, d)}, got {m.shape}")
+        # (c, i, j) in C order is element (j, i) column-major; the library requires exact symmetry, so the two agree
+        check(lib().mcmcgpu_run_set_dense_metric(self.h, dptr(m), 1 if m.ndim == 3 else 0))
+
+    def get_dense_metric(self):
+        """(nchains, d, d) current dense inverse metric"""
+        out = np.empty((self.C, self.d, self.d))
+        check(lib().mcmcgpu_run_get_dense_metric(self.h, dptr(out)))
+        return np.ascontiguousarray(out.transpose(0, 2, 1))               # column-major blocks -> [c, i, j]
 
     def fetch(self, samples=True, grads=None, accept=True, logtarget=None, out=None):
         grads = self.store_grad if grads is None else grads

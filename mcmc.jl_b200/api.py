@@ -305,30 +305,49 @@ class NUTS(_Sampler):
     shrinkage / t0 / step are the dual averaging's gamma / t0 / kappa (HMCDA's).  The mass matrix is the identity unless
     inv_metric gives a diagonal inverse metric, (d,) for every chain or (nchains, d) per chain; adapt_metric=True adapts
     each chain's diagonal metric during warm-up in Stan's windows (init_buffer / term_buffer / window, Stan's defaults),
-    starting from inv_metric or ones.  Runs on the wave engine; the model's scale is not used."""
+    starting from inv_metric or ones.  metric="dense" makes the metric a full matrix (Stan's dense_e): inv_metric is then
+    (d, d) for every chain or (nchains, d, d) per chain, symmetric and positive definite, and the identity when None;
+    adapt_metric=True adapts it from each chain's Welford covariance in the same windows.  Runs on the wave engine; the
+    model's scale is not used."""
 
     def __init__(self, rate=0.6, maxdoublings=10, shrinkage=0.05, t0=10.0, step=0.75, inv_metric=None, adapt_metric=False,
-                 init_buffer=75, term_buffer=50, window=25):
+                 init_buffer=75, term_buffer=50, window=25, metric="diag"):
         assert 0.0 < rate < 1.0, f"Target acceptance rate ({rate}) should be between 0 and 1"
         assert isinstance(maxdoublings, (int, np.integer)) and 1 <= maxdoublings <= 10, \
             f"maxdoublings parameter of NUTS sampler ({maxdoublings}) must be an integer in 1..10"
         assert shrinkage > 0.0, f"shrinkage parameter of NUTS sampler ({shrinkage}) must be positive"
         assert t0 >= 0, f"t0 parameter of NUTS sampler ({t0}) must be non-negative"
-        if inv_metric is not None:
+        assert metric in ("diag", "dense"), f"metric of NUTS sampler must be 'diag' or 'dense', got {metric!r}"
+        if inv_metric is not None and metric == "diag":
             inv_metric = np.array(inv_metric, dtype=np.float64)
             assert inv_metric.ndim in (1, 2) and inv_metric.size > 0, \
                 f"inv_metric of NUTS sampler must be (d,) or (nchains, d), got shape {inv_metric.shape}"
             assert np.all(np.isfinite(inv_metric)) and np.all(inv_metric > 0), "inv_metric of NUTS sampler must be positive and finite"
+        elif inv_metric is not None:
+            inv_metric = np.array(inv_metric, dtype=np.float64)
+            assert inv_metric.ndim in (2, 3) and inv_metric.size > 0 and inv_metric.shape[-1] == inv_metric.shape[-2], \
+                f"dense inv_metric of NUTS sampler must be (d, d) or (nchains, d, d), got shape {inv_metric.shape}"
+            assert np.all(np.isfinite(inv_metric)), "dense inv_metric of NUTS sampler must be finite"
+            assert np.array_equal(inv_metric, np.swapaxes(inv_metric, -1, -2)), "dense inv_metric of NUTS sampler must be symmetric"
+            try:
+                np.linalg.cholesky(inv_metric)
+            except np.linalg.LinAlgError:
+                raise AssertionError("dense inv_metric of NUTS sampler must be positive definite") from None
         for name, v, lo in (("init_buffer", init_buffer, 0), ("term_buffer", term_buffer, 0), ("window", window, 1)):
             assert isinstance(v, (int, np.integer)) and v >= lo, f"{name} of NUTS sampler ({v}) must be an integer >= {lo}"
         self.rate, self.maxdoublings, self.shrinkage, self.t0, self.step = rate, int(maxdoublings), shrinkage, t0, step
-        self.inv_metric, self.adapt_metric = inv_metric, bool(adapt_metric)
+        self.inv_metric, self.adapt_metric, self.metric = inv_metric, bool(adapt_metric), metric
         self.init_buffer, self.term_buffer, self.window = int(init_buffer), int(term_buffer), int(window)
         self.tuner = None
 
     def _set_metric(self, drun, offset, nchains):
         """the metric calls of a run of chains offset .. offset + drun.C - 1 of nchains (none with the defaults)"""
-        if self.inv_metric is not None:
+        if self.metric == "dense":
+            m = self.inv_metric
+            assert m is None or m.ndim == 2 or m.shape[0] == nchains, \
+                f"dense inv_metric of NUTS sampler has {m.shape[0]} matrices for {nchains} chains"
+            drun.set_dense_metric(m if m is None or m.ndim == 2 else m[offset:offset + drun.C])
+        elif self.inv_metric is not None:
             assert self.inv_metric.ndim == 1 or self.inv_metric.shape[0] == nchains, \
                 f"inv_metric of NUTS sampler has {self.inv_metric.shape[0]} rows for {nchains} chains"
             drun.set_metric(self.inv_metric if self.inv_metric.ndim == 1 else self.inv_metric[offset:offset + drun.C])
@@ -520,7 +539,7 @@ class MCMCChainBatch:
             eps, leaps = self.diag()
             diags["epsilon"] = eps[i]
             diags["ndoublings"] = np.floor(np.log2(leaps[i])).astype(np.int64) + 1    # the tree of 2^(n-1) .. 2^n - 1 leapfrogs
-            if s.inv_metric is not None or s.adapt_metric:
+            if s.inv_metric is not None or s.adapt_metric or s.metric == "dense":
                 diags["inv_metric"] = self.inv_metric()[i]
         g = a.get("grads")
         return MCMCChain(self.range, a["samples"][i], None if g is None else g[i], diags, self.task, self.runTime,
@@ -536,9 +555,11 @@ class MCMCChainBatch:
         return self._diag
 
     def inv_metric(self):
-        """(C, d) diagonal inverse metric of every chain at the end of the run (NUTS; ones for the identity)"""
+        """the inverse metric of every chain at the end of the run (NUTS): (C, d) diagonal (ones for the identity), or
+        (C, d, d) for a dense metric"""
         if getattr(self, "_minv", None) is None:
-            self._minv = self._run.get_metric()
+            dense = getattr(self.task.sampler, "metric", "diag") == "dense"
+            self._minv = self._run.get_dense_metric() if dense else self._run.get_metric()
         return self._minv
 
     def stats(self, vtype="imse", **kw):

@@ -947,6 +947,7 @@ int32_t mcmcgpu_run_set_metric(mcmcgpu_run* R, const double* inv_metric, int32_t
   if (!R || !inv_metric) return fail(MCMCGPU_E_ARG, "NULL argument");
   if (R->s.kind != MCMCGPU_NUTS) return fail(MCMCGPU_E_ARG, "a metric applies to NUTS");
   if (R->started) return fail(MCMCGPU_E_STATE, "the metric must be set before the first execute");
+  if (R->nuts.A) return fail(MCMCGPU_E_ARG, "the run has a dense metric (mcmcgpu_run_set_dense_metric)");
   const int64_t C = R->C, d = R->d, n = per_chain ? C * d : d;
   for (int64_t k = 0; k < n; k++)
     if (!(std::isfinite(inv_metric[k]) && inv_metric[k] > 0)) return fail(MCMCGPU_E_ARG, "every inverse metric entry must be finite and > 0");
@@ -965,16 +966,26 @@ int32_t mcmcgpu_run_set_metric_adaptation(mcmcgpu_run* R, int64_t init_buffer, i
   if (step0_in_warmup(R, R->step0)) return fail(MCMCGPU_E_ARG, "metric adaptation cannot start inside the warm-up (set_state step0)");
   CU(use_ctx(R->m->ctx));
   NutsState& T = R->nuts;
-  if (!T.minv) {
+  const bool dense = T.A != nullptr;
+  const int64_t dd = R->d * R->d;
+  if (!dense && !T.minv) {
     std::vector<double> ones((size_t)(R->C * R->d), 1.0);
     int rc = upload_metric(R, ones.data());
     if (rc) return rc;
+  }
+  if (dense && T.a_ld == 1) {      // every chain adapts its own copy of the shared starting matrix and its factor
+    double *A = nullptr, *L = nullptr;
+    CU(R->alloc(&A, (size_t)(dd * R->Cp), false));
+    CU(R->alloc(&L, (size_t)(dd * R->Cp), false));
+    CU(broadcast_to_chain_minor(T.A, A, dd, R->C, R->Cp, R->m->ctx->stream));
+    CU(broadcast_to_chain_minor(T.L, L, dd, R->C, R->Cp, R->m->ctx->stream));
+    T.A = A; T.L = L; T.a_ld = R->Cp;
   }
   int64_t lo, hi;
   const std::vector<int64_t> ends = metric_windows(R->r.first - 2, init_buffer, term_buffer, window, &lo, &hi);
   if (!T.wf_mean) {
     CU(R->alloc(&T.wf_mean, (size_t)(R->d * R->Cp)));
-    CU(R->alloc(&T.wf_m2, (size_t)(R->d * R->Cp)));
+    CU(R->alloc(&T.wf_m2, (size_t)((dense ? dd : R->d) * R->Cp)));
     CU(R->alloc(&T.wf_n, (size_t)R->Cp));
     CU(R->alloc(&T.da_eps0, (size_t)R->Cp));
     CU(R->alloc(&T.da_i0, (size_t)R->Cp));
@@ -992,6 +1003,7 @@ int32_t mcmcgpu_run_set_metric_adaptation(mcmcgpu_run* R, int64_t init_buffer, i
 int32_t mcmcgpu_run_get_metric(mcmcgpu_run* R, double* out_inv_metric) {
   if (!R || !out_inv_metric) return fail(MCMCGPU_E_ARG, "NULL argument");
   if (R->s.kind != MCMCGPU_NUTS) return fail(MCMCGPU_E_ARG, "a metric applies to NUTS");
+  if (R->nuts.A) return fail(MCMCGPU_E_ARG, "the run has a dense metric: use mcmcgpu_run_get_dense_metric");
   if (!R->nuts.minv) {
     std::fill(out_inv_metric, out_inv_metric + R->C * R->d, 1.0);
     return MCMCGPU_OK;
@@ -1004,6 +1016,84 @@ int32_t mcmcgpu_run_get_metric(mcmcgpu_run* R, double* out_inv_metric) {
   CU(transpose_to_chain_major(R->nuts.minv, tmp, 0, R->C, R->d, R->Cp, st));
   CU(cudaMemcpyAsync(out_inv_metric, tmp, sizeof(double) * (size_t)(R->C * R->d), cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
+  return MCMCGPU_OK;
+}
+
+// A dense metric: every matrix finite and exactly symmetric on the host, then positive definite by the device Cholesky
+// that nuts_kernel uses (the factor it leaves is the run's L).  Being symmetric, a chain's column-major d x d block is also
+// its row-major one, which is the device layout.  A shared matrix is stored once (a_ld = 1) and read by every chain.
+int32_t mcmcgpu_run_set_dense_metric(mcmcgpu_run* R, const double* inv_metric, int32_t per_chain) {
+  if (!R) return fail(MCMCGPU_E_ARG, "run is NULL");
+  if (R->s.kind != MCMCGPU_NUTS) return fail(MCMCGPU_E_ARG, "a metric applies to NUTS");
+  if (R->started) return fail(MCMCGPU_E_STATE, "the metric must be set before the first execute");
+  if (R->adapt_metric) return fail(MCMCGPU_E_ARG, "set the dense metric before mcmcgpu_run_set_metric_adaptation");
+  if (R->nuts.minv) return fail(MCMCGPU_E_ARG, "the run has a diagonal metric (mcmcgpu_run_set_metric)");
+  const int64_t d = R->d, dd = d * d, Cp = R->Cp;
+  std::vector<double> ident;
+  if (!inv_metric) {
+    ident.assign((size_t)dd, 0.0);
+    for (int64_t j = 0; j < d; j++) ident[(size_t)(j * d + j)] = 1.0;
+    inv_metric = ident.data(); per_chain = 0;
+  }
+  const int64_t nm = per_chain ? R->C : 1, ld = per_chain ? Cp : 1;
+  for (int64_t c = 0; c < nm; c++)
+    for (int64_t j = 0; j < d; j++)
+      for (int64_t i = 0; i < d; i++) {
+        const double x = inv_metric[c * dd + j * d + i];
+        if (!std::isfinite(x)) return fail(MCMCGPU_E_ARG, "every dense inverse metric entry must be finite");
+        if (x != inv_metric[c * dd + i * d + j]) return fail(MCMCGPU_E_ARG, "every dense inverse metric must be exactly symmetric");
+      }
+  CU(use_ctx(R->m->ctx));
+  cudaStream_t st = R->m->ctx->stream;
+  double *A = nullptr, *L = nullptr, *tmp = nullptr;
+  int32_t* bad = nullptr;
+  DevBufs bufs;
+  CU(R->alloc(&A, (size_t)(dd * ld), false));
+  CU(R->alloc(&L, (size_t)(dd * ld)));
+  if (per_chain) {
+    CU(bufs.up(&tmp, inv_metric, (size_t)(nm * dd), st));
+    CU(transpose_to_chain_minor(tmp, A, nm, dd, Cp, st));
+  } else {
+    CU(cudaMemcpyAsync(A, inv_metric, sizeof(double) * (size_t)dd, cudaMemcpyHostToDevice, st));
+  }
+  CU(bufs.get(&bad, (size_t)nm, st, false));
+  CU(launch_dense_factor(A, L, d, nm, ld, bad, st));
+  std::vector<int32_t> hbad((size_t)nm);
+  CU(cudaMemcpyAsync(hbad.data(), bad, sizeof(int32_t) * (size_t)nm, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  for (int32_t b : hbad)
+    if (b) return fail(MCMCGPU_E_ARG, "every dense inverse metric must be positive definite (its Cholesky factorisation failed)");
+  NutsState& T = R->nuts;
+  if (!T.v[0]) {
+    CU(R->alloc(&T.v[0], (size_t)(d * Cp), false));
+    CU(R->alloc(&T.v[1], (size_t)(d * Cp), false));
+  }
+  T.A = A; T.L = L; T.a_ld = ld;
+  return MCMCGPU_OK;
+}
+
+int32_t mcmcgpu_run_get_dense_metric(mcmcgpu_run* R, double* out) {
+  if (!R || !out) return fail(MCMCGPU_E_ARG, "NULL argument");
+  if (R->s.kind != MCMCGPU_NUTS || !R->nuts.A) return fail(MCMCGPU_E_ARG, "the run has no dense metric");
+  CU(use_ctx(R->m->ctx));
+  cudaStream_t st = R->m->ctx->stream;
+  const NutsState& T = R->nuts;
+  const int64_t C = R->C, d = R->d, dd = d * d;
+  if (T.a_ld == 1) {
+    CU(cudaMemcpyAsync(out, T.A, sizeof(double) * (size_t)dd, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    for (int64_t c = 1; c < C; c++) std::copy(out, out + dd, out + c * dd);
+  } else {
+    double* tmp = nullptr;
+    DevBufs bufs;
+    CU(bufs.get(&tmp, (size_t)(C * dd), st, false));
+    CU(transpose_to_chain_major(T.A, tmp, 0, C, dd, R->Cp, st));
+    CU(cudaMemcpyAsync(out, tmp, sizeof(double) * (size_t)(C * dd), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+  }
+  for (int64_t c = 0; c < C; c++)            // row-major (device) to column-major: an adapted A is not exactly symmetric
+    for (int64_t j = 0; j < d; j++)
+      for (int64_t k = j + 1; k < d; k++) std::swap(out[c * dd + j * d + k], out[c * dd + k * d + j]);
   return MCMCGPU_OK;
 }
 

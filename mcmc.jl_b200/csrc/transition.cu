@@ -815,9 +815,14 @@ __global__ void __launch_bounds__(CO_CHAINS * CO_GROUPS, 2) transition_coop_kern
 // of doubling j from NUTS_TREE_BLOCK + 2j, its merge from NUTS_TREE_BLOCK + 2j + 1, candidate choice of the step's leaf
 // k (0-based) from NUTS_LEAF_BLOCK + k.  One thread per chain; every array is chain-minor, so a warp's accesses coalesce.
 //
-// MET: a diagonal inverse metric minv = M^-1 (NutsState::minv).  It enters as p = z / sqrt(minv), K = 0.5 sum (minv p) p,
-// theta += e (minv m) and the U-turn dots delta . (minv p); with MET = false every one of these is the identity's operation
-// and minv is never loaded.  (z / 1, 1 * p and 1 * m are exact, so an all-ones metric gives the identity's bits.)
+// MET: the kind of inverse metric M^-1.  NUTS_DIAG: a diagonal minv (NutsState::minv).  It enters as p = z / sqrt(minv),
+// K = 0.5 sum (minv p) p, theta += e (minv m) and the U-turn dots delta . (minv p); with NUTS_UNIT every one of these is
+// the identity's operation and minv is never loaded.  (z / 1, 1 * p and 1 * m are exact, so an all-ones metric gives the
+// identity's bits.)  NUTS_DENSE: a full matrix A and its lower Cholesky factor L (NutsState::A, L): p = L^-T z by back
+// substitution, v = A m (k ascending from 0.0), K = 0.5 sum_j v_j m_j, theta += e v with v = A m taken after the momentum
+// half-step, and the U-turn dots delta . v with v stored for both tree ends (NutsState::v) and every checkpoint (ck_p).
+// A diagonal A then computes exactly the diagonal metric's products (the zeros add nothing), so it gives their bits.
+constexpr int NUTS_UNIT = 0, NUTS_DIAG = 1, NUTS_DENSE = 2;
 
 // minv_j * x, or x itself for the identity metric
 template <bool MET>
@@ -873,7 +878,93 @@ __device__ void nuts_adapt_metric(const WaveArgs& W, const int64_t c, int64_t i,
   W.da_dual[c] = 1.0; W.da_dualH[c] = 0.0;
 }
 
-template <bool MET>
+// v_j = sum_k A[j][k] x_k from 0.0, k ascending; Ac = chain c's A (element (j, k) at (j d + k) ld), x chain-minor
+__device__ __forceinline__ double dense_row(const double* Ac, int64_t ld, int64_t j, const double* x, int64_t d, int64_t Cp,
+                                           int64_t c) {
+  double s = 0.0;
+  for (int64_t k = 0; k < d; k++) s += Ac[(j * d + k) * ld] * x[k * Cp + c];
+  return s;
+}
+
+// the position half of a leapfrog with a dense metric: q_j = th_j + e (A m)_j
+__device__ __forceinline__ void dense_position(const double* Ac, int64_t ld, const double* th, const double* m, double* q, double e,
+                                               int64_t d, int64_t Cp, int64_t c) {
+  for (int64_t j = 0; j < d; j++) {
+    double p = th[j * Cp + c];
+    p += e * dense_row(Ac, ld, j, m, d, Cp, c);
+    q[j * Cp + c] = p;
+  }
+}
+
+// Lower Cholesky factor l of the matrix whose lower triangle a holds (element (i, j) at (i d + j) ld), in the pinned order:
+// for j = 0 .. d-1, s = a_jj, s -= l_jk l_jk for k < j ascending, l_jj = sqrt(s); for i > j, t = a_ij, t -= l_ik l_jk for
+// k < j ascending, l_ij = t / l_jj.  False (l partly written) when a pivot s is not finite and > 0.
+__device__ bool dense_cholesky(const double* a, double* l, int64_t d, int64_t ld) {
+  for (int64_t j = 0; j < d; j++) {
+    double s = a[(j * d + j) * ld];
+    for (int64_t k = 0; k < j; k++) s -= l[(j * d + k) * ld] * l[(j * d + k) * ld];
+    if (!(s > 0.0 && isfinite(s))) return false;
+    const double ljj = sqrt(s);
+    l[(j * d + j) * ld] = ljj;
+    for (int64_t i = j + 1; i < d; i++) {
+      double t = a[(i * d + j) * ld];
+      for (int64_t k = 0; k < j; k++) t -= l[(i * d + k) * ld] * l[(j * d + k) * ld];
+      l[(i * d + j) * ld] = t / ljj;
+    }
+  }
+  return true;
+}
+
+// Dense metric adaptation (Stan's covar_adaptation::learn_covariance with welford_covar_estimator), in nuts_adapt_metric's
+// order: the step's final sample x joins the window's sums (n += 1, delta = x - mean, mean += delta / n, then
+// m2[a][b] += (x_a - mean_a) delta_b with the new mean: full, not symmetrised, as Stan's estimator).  At a window end
+// A = (n / (n + 5)) cov + 1e-3 (5 / (n + 5)) I with cov = m2 / (n - 1) (n <= 1: the current A), built in place of m2, and
+// L = chol(A); if that Cholesky fails the chain keeps its A, whose factor is recomputed bit for bit.  Then the sums reset
+// and the dual averaging restarts as for the diagonal metric.  A, L and m2 are per chain here (ld = Cp).
+__device__ void nuts_adapt_dense(const WaveArgs& W, const int64_t c, int64_t i, double eps) {
+  const NutsState& T = W.nuts;
+  const int64_t d = W.M.d, Cp = W.R.Cp;
+  const double* x = W.cur_pars;
+  if (i >= T.win_lo && i <= T.win_hi) {
+    const double n = (double)(T.wf_n[c] + 1);
+    T.wf_n[c] += 1;
+    for (int64_t a = 0; a < d; a++) {
+      const double xa = x[a * Cp + c], ma = T.wf_mean[a * Cp + c];
+      const double ra = xa - (ma + (xa - ma) / n);                      // x_a minus its updated mean
+      for (int64_t b = 0; b < d; b++) T.wf_m2[(a * d + b) * Cp + c] += ra * (x[b * Cp + c] - T.wf_mean[b * Cp + c]);
+    }
+    for (int64_t j = 0; j < d; j++) {
+      const double xj = x[j * Cp + c];
+      double mean = T.wf_mean[j * Cp + c];
+      mean += (xj - mean) / n;
+      T.wf_mean[j * Cp + c] = mean;
+    }
+  }
+  bool end = false;
+  for (int k = 0; k < T.n_win; k++) end |= T.win_end[k] == i;
+  if (!end) return;
+  const double n = (double)T.wf_n[c];
+  for (int64_t a = 0; a < d; a++)
+    for (int64_t b = 0; b < d; b++) {
+      const int64_t at = (a * d + b) * Cp + c;
+      const double cov = n > 1.0 ? T.wf_m2[at] / (n - 1.0) : T.A[at];
+      double an = (n / (n + 5.0)) * cov;
+      if (a == b) an = an + 1e-3 * (5.0 / (n + 5.0));
+      T.wf_m2[at] = an;
+    }
+  if (dense_cholesky(T.wf_m2 + c, T.L + c, d, Cp)) {
+    for (int64_t k = 0; k < d * d; k++) T.A[k * Cp + c] = T.wf_m2[k * Cp + c];
+  } else {
+    dense_cholesky(T.A + c, T.L + c, d, Cp);
+  }
+  for (int64_t k = 0; k < d * d; k++) T.wf_m2[k * Cp + c] = 0.0;
+  for (int64_t j = 0; j < d; j++) T.wf_mean[j * Cp + c] = 0.0;
+  T.wf_n[c] = 0;
+  T.da_eps0[c] = eps; T.da_i0[c] = i;
+  W.da_dual[c] = 1.0; W.da_dualH[c] = 0.0;
+}
+
+template <int MET>
 __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
   const RunnerDev& R = W.R;
   const SamplerDev& S = W.S;
@@ -913,7 +1004,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       W.cur_grad[j * Cp + c] = fin_grad(F, M, q, part, ns, Cp, c, j);
     }
     if (!W.restore_da) { W.da_leapstep[c] = 1.0; W.da_dual[c] = 1.0; W.da_dualH[c] = 0.0; }   // eps0 = 1, as HMCDA
-    if constexpr (MET) if (T.win_end) { T.da_eps0[c] = 1.0; T.da_i0[c] = 0; }
+    if constexpr (MET != NUTS_UNIT) if (T.win_end) { T.da_eps0[c] = 1.0; T.da_i0[c] = 0; }
     i = W.step0 + 1;
     begin = true;
   } else {   // PH_NUTS: leaf `leaf` of the subtree of doubling jd has been evaluated at q
@@ -929,9 +1020,16 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       const double gj = fin_grad(F, M, q, part, ns, Cp, c, j);
       double m = W.mom[j * Cp + c];
       m += (0.5 * gj) * e;
-      mm += nuts_mv<MET>(T.minv, j * Cp + c, m) * m;
+      if constexpr (MET != NUTS_DENSE) mm += nuts_mv<MET == NUTS_DIAG>(T.minv, j * Cp + c, m) * m;
       th_v[j * Cp + c] = q[j * Cp + c]; p_v[j * Cp + c] = m; g_v[j * Cp + c] = gj;
     }
+    if constexpr (MET == NUTS_DENSE)                                    // v = A p of the new end, K = 0.5 v . p
+      for (int64_t j = 0; j < d; j++) {
+        const double vj = dense_row(T.A + (T.a_ld == 1 ? 0 : c), T.a_ld, j, p_v, d, Cp, c);
+        T.v[side][j * Cp + c] = vj;
+        mm += vj * p_v[j * Cp + c];
+      }
+    const double* w_v = MET == NUTS_DENSE ? T.v[side] : p_v;            // what the U-turn dots take: A p, or p
     const double H = -F.lt + 0.5 * mm;                                  // update! HMC.jl:91
     const double H0 = W.H0[c], lu0 = T.log_u0[c];
     const int k = T.leaps[c];
@@ -950,21 +1048,26 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
     }
     const int64_t slot = d * Cp;
     for (int r = 1; s && r <= jd && (leaf & ((1 << r) - 1)) == 0; r++)        // U-turn checks of the blocks this leaf closes
-      s = nuts_no_uturn<MET>(th_v, p_v, T.ck_th + (r - 1) * slot, T.ck_p + (r - 1) * slot, v, T.minv, d, Cp, c);
+      s = nuts_no_uturn<MET == NUTS_DIAG>(th_v, w_v, T.ck_th + (r - 1) * slot, T.ck_p + (r - 1) * slot, v, T.minv, d, Cp, c);
     bool open = false;
     if (s && leaf < (1 << jd)) {                                        // next leaf of this subtree
       for (int r = 1; r <= jd && ((leaf - 1) & ((1 << r) - 1)) == 0; r++)     // checkpoints of the blocks this leaf opens
         for (int64_t j = 0; j < d; j++) {
           T.ck_th[(r - 1) * slot + j * Cp + c] = th_v[j * Cp + c];
-          T.ck_p[(r - 1) * slot + j * Cp + c] = p_v[j * Cp + c];
+          T.ck_p[(r - 1) * slot + j * Cp + c] = w_v[j * Cp + c];
         }
       for (int64_t j = 0; j < d; j++) {                                 // HMC.jl:95-96 from the end just reached
         double m = p_v[j * Cp + c];
         m += (0.5 * g_v[j * Cp + c]) * e;
-        double p = th_v[j * Cp + c];
-        p += e * nuts_mv<MET>(T.minv, j * Cp + c, m);
-        W.mom[j * Cp + c] = m; q[j * Cp + c] = p;
+        if constexpr (MET == NUTS_DENSE) {
+          W.mom[j * Cp + c] = m;
+        } else {
+          double p = th_v[j * Cp + c];
+          p += e * nuts_mv<MET == NUTS_DIAG>(T.minv, j * Cp + c, m);
+          W.mom[j * Cp + c] = m; q[j * Cp + c] = p;
+        }
       }
+      if constexpr (MET == NUTS_DENSE) dense_position(T.A + (T.a_ld == 1 ? 0 : c), T.a_ld, th_v, W.mom, q, e, d, Cp, c);
       T.leaf[c] = leaf + 1;
       return nev;
     } else if (s) {                                                     // the subtree is complete: merge it into the tree
@@ -975,7 +1078,8 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
         T.moved[c] = 1;
       }
       T.n[c] = n + nsub;
-      open = jd + 1 < S.nleaps && nuts_no_uturn<MET>(T.th[1], T.p[1], T.th[0], T.p[0], 1.0, T.minv, d, Cp, c);
+      open = jd + 1 < S.nleaps && nuts_no_uturn<MET == NUTS_DIAG>(T.th[1], MET == NUTS_DENSE ? T.v[1] : T.p[1], T.th[0],
+                                                                   MET == NUTS_DENSE ? T.v[0] : T.p[0], 1.0, T.minv, d, Cp, c);
     }
     if (open) {
       doubling = true; jnext = jd + 1;
@@ -985,10 +1089,11 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       if (i < burnin) {
         double eps0 = 1.0;
         int64_t i0 = 0;
-        if constexpr (MET) if (T.win_end) { eps0 = T.da_eps0[c]; i0 = T.da_i0[c]; }
+        if constexpr (MET != NUTS_UNIT) if (T.win_end) { eps0 = T.da_eps0[c]; i0 = T.da_i0[c]; }
         const DaStep a = da_adapt(S, i, pacc, W.da_dual[c], W.da_dualH[c], 10.0 * eps0, i0);
         W.da_dual[c] = a.dual; W.da_dualH[c] = a.dualH; W.da_leapstep[c] = a.leapstep;
-        if constexpr (MET) if (T.win_end) nuts_adapt_metric(W, c, i, a.leapstep);
+        if constexpr (MET == NUTS_DIAG) if (T.win_end) nuts_adapt_metric(W, c, i, a.leapstep);
+        if constexpr (MET == NUTS_DENSE) if (T.win_end) nuts_adapt_dense(W, c, i, a.leapstep);
       } else {
         W.da_leapstep[c] = W.da_dual[c];
       }
@@ -1019,12 +1124,27 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
         const int64_t j = jb + t;
         if (j >= d) break;
         double z = t ? z1 : z0;
-        if constexpr (MET) z = z / sqrt(T.minv[j * Cp + c]);                  // p = z / sqrt(minv)
-        mm += nuts_mv<MET>(T.minv, j * Cp + c, z) * z;
+        if constexpr (MET == NUTS_DIAG) z = z / sqrt(T.minv[j * Cp + c]);     // p = z / sqrt(minv)
+        if constexpr (MET != NUTS_DENSE) mm += nuts_mv<MET == NUTS_DIAG>(T.minv, j * Cp + c, z) * z;
         const double pj = W.cur_pars[j * Cp + c], gj = W.cur_grad[j * Cp + c];
         T.th[0][j * Cp + c] = pj; T.th[1][j * Cp + c] = pj;
         T.p[0][j * Cp + c] = z; T.p[1][j * Cp + c] = z;
         T.g[0][j * Cp + c] = gj; T.g[1][j * Cp + c] = gj;
+      }
+    }
+    if constexpr (MET == NUTS_DENSE) {   // p = L^-T z by back substitution (Stan's llt().matrixU().solve), v = A p, K = 0.5 v . p
+      const double* Lc = T.L + (T.a_ld == 1 ? 0 : c);
+      double* p0 = T.p[0];
+      for (int64_t j = d - 1; j >= 0; j--) {
+        double s = p0[j * Cp + c];
+        for (int64_t k = j + 1; k < d; k++) s -= Lc[(k * d + j) * T.a_ld] * p0[k * Cp + c];
+        p0[j * Cp + c] = s / Lc[(j * d + j) * T.a_ld];
+      }
+      for (int64_t j = 0; j < d; j++) {
+        const double pj = p0[j * Cp + c];
+        const double vj = dense_row(T.A + (T.a_ld == 1 ? 0 : c), T.a_ld, j, p0, d, Cp, c);
+        mm += vj * pj;
+        T.p[1][j * Cp + c] = pj; T.v[0][j * Cp + c] = vj; T.v[1][j * Cp + c] = vj;
       }
     }
     W.H0[c] = -W.cur_lt[c] + 0.5 * mm;                                  // update! HMC.jl:91
@@ -1043,10 +1163,15 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
     for (int64_t j = 0; j < d; j++) {
       double m = p_v[j * Cp + c];
       m += (0.5 * g_v[j * Cp + c]) * e;                                 // HMC.jl:95
-      double p = th_v[j * Cp + c];
-      p += e * nuts_mv<MET>(T.minv, j * Cp + c, m);                     // HMC.jl:96
-      W.mom[j * Cp + c] = m; q[j * Cp + c] = p;
+      if constexpr (MET == NUTS_DENSE) {
+        W.mom[j * Cp + c] = m;
+      } else {
+        double p = th_v[j * Cp + c];
+        p += e * nuts_mv<MET == NUTS_DIAG>(T.minv, j * Cp + c, m);      // HMC.jl:96
+        W.mom[j * Cp + c] = m; q[j * Cp + c] = p;
+      }
     }
+    if constexpr (MET == NUTS_DENSE) dense_position(T.A + (T.a_ld == 1 ? 0 : c), T.a_ld, th_v, W.mom, q, e, d, Cp, c);   // HMC.jl:96
     W.need_ll[c] = 1;
     W.phase[c] = PH_NUTS;
   }
@@ -1054,7 +1179,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
 }
 
 constexpr int NUTS_THREADS = 128;
-template <bool MET>
+template <int MET>
 __global__ void __launch_bounds__(NUTS_THREADS) nuts_kernel(const WaveArgs W) {
   if (!W.resume && *W.remaining == 0) return;
   const int64_t c = (int64_t)blockIdx.x * NUTS_THREADS + threadIdx.x;
@@ -1066,8 +1191,9 @@ __global__ void __launch_bounds__(NUTS_THREADS) nuts_kernel(const WaveArgs W) {
 cudaError_t launch_transition(const WaveArgs& W, cudaStream_t st) {
   if (W.S.kind == MCMCGPU_NUTS) {
     const unsigned blocks = (unsigned)((W.R.C + NUTS_THREADS - 1) / NUTS_THREADS);
-    if (W.nuts.minv) nuts_kernel<true><<<blocks, NUTS_THREADS, 0, st>>>(W);
-    else nuts_kernel<false><<<blocks, NUTS_THREADS, 0, st>>>(W);
+    if (W.nuts.A) nuts_kernel<NUTS_DENSE><<<blocks, NUTS_THREADS, 0, st>>>(W);
+    else if (W.nuts.minv) nuts_kernel<NUTS_DIAG><<<blocks, NUTS_THREADS, 0, st>>>(W);
+    else nuts_kernel<NUTS_UNIT><<<blocks, NUTS_THREADS, 0, st>>>(W);
     return cudaGetLastError();
   }
   const bool regression = (W.M.family == MCMCGPU_FAM_LINEAR || W.M.family == MCMCGPU_FAM_LOGISTIC || W.M.family == MCMCGPU_FAM_PROBIT);
@@ -1081,6 +1207,16 @@ cudaError_t launch_transition(const WaveArgs& W, cudaStream_t st) {
   return cudaGetLastError();
 }
 
+
+// L = chol(A) for n dense metrics at pitch ld (mcmcgpu_run_set_dense_metric); bad[c] = 1 where a pivot fails
+__global__ void __launch_bounds__(128) dense_factor_kernel(const double* A, double* L, int64_t d, int64_t n, int64_t ld, int32_t* bad) {
+  const int64_t c = (int64_t)blockIdx.x * 128 + threadIdx.x;
+  if (c < n) bad[c] = dense_cholesky(A + c, L + c, d, ld) ? 0 : 1;
+}
+cudaError_t launch_dense_factor(const double* A, double* L, int64_t d, int64_t n, int64_t ld, int32_t* bad, cudaStream_t st) {
+  dense_factor_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(A, L, d, n, ld, bad);
+  return cudaGetLastError();
+}
 
 // ---- RAM (robust adaptive Metropolis) for the wave engine ----------------------------------------------
 __global__ void __launch_bounds__(128) ram_kernel(const WaveArgs W, int init) {
@@ -1436,6 +1572,17 @@ cudaError_t launch_philox_dump(uint64_t seed, int64_t chain_offset, int64_t C, i
 __global__ void fill_kernel(double* p, double v, int64_t n) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) p[i] = v;
+}
+__global__ void broadcast_kernel(const double* src, double* dst, int64_t K, int64_t C, int64_t Cp) {
+  const int64_t n = K * C;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x)
+    dst[(t / C) * Cp + t % C] = src[t / C];
+}
+cudaError_t broadcast_to_chain_minor(const double* src, double* dst, int64_t K, int64_t C, int64_t Cp, cudaStream_t st) {
+  const int64_t n = K * C;
+  const int64_t blocks = (n + 255) / 256;
+  broadcast_kernel<<<(unsigned)(blocks < 8192 ? blocks : 8192), 256, 0, st>>>(src, dst, K, C, Cp);
+  return cudaGetLastError();
 }
 cudaError_t launch_fill(double* p, double v, int64_t n, cudaStream_t st) {
   fill_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(p, v, n);

@@ -37,7 +37,13 @@ struct NutsState {
   int64_t* da_i0;              // [Cp] step of the last restart (the dual averaging counts steps from it)
   const int64_t* win_end;      // [n_win] ascending
   int64_t win_lo, win_hi;
-  int32_t n_win;
+  int32_t n_win;  // dense inverse metric (mcmcgpu_run_set_dense_metric; null A: none).  Element (j, k) of chain c's matrix at
+  // (j*d + k)*a_ld + c with a_ld = Cp, or at (j*d + k) for one matrix every chain reads (a_ld = 1: a fixed shared metric).
+  // With adaptation A and L are per chain and wf_m2 is [d*d][Cp] (the full Welford sum of cross products).
+  double* A;                   // M^-1
+  double* L;                   // lower Cholesky factor of A (the upper triangle is not used)
+  double* v[2];                // [d][Cp] A p of each tree end; with a dense metric ck_p holds A p instead of p
+  int64_t a_ld;
 };
 
 struct WaveArgs {
@@ -101,5 +107,8 @@ cudaError_t transpose_to_chain_major_u8(const uint8_t* in, uint8_t* out, int64_t
 cudaError_t launch_philox_dump(uint64_t seed, int64_t chain_offset, int64_t C, int64_t d, int64_t last,
                                double* normals /*[C][last+1][d]*/, double* uniforms /*[C][last+1]*/, cudaStream_t st);
 cudaError_t launch_fill(double* p, double v, int64_t n, cudaStream_t st);
+// dense metric: L = chol(A) of n matrices at pitch ld, bad[c] = 1 where that fails; src [K] copied to every chain of dst [K][Cp]
+cudaError_t launch_dense_factor(const double* A, double* L, int64_t d, int64_t n, int64_t ld, int32_t* bad, cudaStream_t st);
+cudaError_t broadcast_to_chain_minor(const double* src, double* dst, int64_t K, int64_t C, int64_t Cp, cudaStream_t st);
 
 }  // namespace mg

@@ -83,8 +83,12 @@ samplercfg(s::NUTS)  = SamplerCfg(5, s.maxdoublings, 0., s.rate, 0., s.shrinkage
 # NUTS's diagonal metric on a run handle (mcmcgpu_run_create), before its first execute.  The NUTS type carries
 #   invmetric::Union(Nothing, Array{Float64})   # d, or d x nchains; nothing = the identity
 #   adaptmetric::Bool; initbuffer::Int; termbuffer::Int; window::Int   # Stan's windows, defaults 75 / 50 / 25
+#   metric::Symbol                              # :diag, or :dense with invmetric d x d / d x d x nchains (nothing = I)
 function nuts_metric!(run::Ptr{Void}, s::NUTS)
-  if s.invmetric != nothing
+  if s.metric == :dense
+    check(ccall((:mcmcgpu_run_set_dense_metric, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}, Int32),
+                run, s.invmetric == nothing ? C_NULL : s.invmetric, s.invmetric != nothing && ndims(s.invmetric) == 3 ? 1 : 0))
+  elseif s.invmetric != nothing
     check(ccall((:mcmcgpu_run_set_metric, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}, Int32),
                 run, s.invmetric, ndims(s.invmetric) == 2 ? 1 : 0))
   end
@@ -97,6 +101,12 @@ end
 function nuts_metric(run::Ptr{Void}, d::Int, nchains::Int)
   out = Array(Float64, d, nchains)
   check(ccall((:mcmcgpu_run_get_metric, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}), run, out))
+  out
+end
+# the d x d x nchains dense inverse metric of a run with metric = :dense
+function nuts_dense_metric(run::Ptr{Void}, d::Int, nchains::Int)
+  out = Array(Float64, d, d, nchains)
+  check(ccall((:mcmcgpu_run_get_dense_metric, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}), run, out))
   out
 end
 

@@ -53,17 +53,23 @@ extern "C" {
 #define MCMCGPU_HMC 2
 #define MCMCGPU_HMCDA 3
 #define MCMCGPU_RAM 4          /* src/samplers/RAM.jl:24-36: scale, rate (robust adaptive Metropolis); d <= 8 fused, d <= 128 wave */
-/* No-U-Turn sampler: slice NUTS with dual averaging (Hoffman & Gelman 2014, Algorithms 3 and 6), with the identity, a
- * diagonal or a dense mass matrix, fixed (mcmcgpu_run_set_metric / _set_dense_metric) or adapted per chain in Stan's
- * warm-up windows (mcmcgpu_run_set_metric_adaptation), engine WAVE only (one leapfrog leaf per chain per wave).  It reads
- * mcmcgpu_sampler_cfg as follows:
+/* No-U-Turn sampler with dual averaging, with the identity, a diagonal or a dense mass matrix, fixed
+ * (mcmcgpu_run_set_metric / _set_dense_metric) or adapted per chain in Stan's warm-up windows
+ * (mcmcgpu_run_set_metric_adaptation), engine WAVE only (one leapfrog leaf per chain per wave).  Two transitions
+ * (mcmcgpu_run_set_nuts_transition): slice NUTS (Hoffman & Gelman 2014, Algorithms 3 and 6; the default) and Stan's
+ * multinomial NUTS (biased progressive sampling, U-turn checks across neighbouring sub-trees, divergences at
+ * H - H0 > 1000).  It reads mcmcgpu_sampler_cfg as follows:
  *   nleaps = maxdoublings (1..10: at most 2^maxdoublings - 1 leapfrogs per step);
- *   rate, shrinkage, t0, step = the dual averaging, HMCDA's rules (the target is the mean acceptance statistic of the
- *   last doubling); scale, len and max_leaps are ignored, and so is the model scale passed to the run.
+ *   rate, shrinkage, t0, step = the dual averaging, HMCDA's rules.  Its target statistic is, for slice NUTS, the mean
+ *   of min(1, exp(H0 - H)) over the last doubling's leaves and, for multinomial NUTS, Stan's accept_stat: the same
+ *   mean over every leaf of the step's trajectory.  scale, len and max_leaps are ignored, and so is the model scale
+ *   passed to the run.
  * fetch_diag returns the step size and the leapfrog count of every kept step (ndoublings = floor(log2(leaps)) + 1);
  * set_state / get_state carry (step size, dual step size, dualH) as for HMCDA.  Not supported: engine FUSED, injected
  * draws, store_rb, a tuner, row-sharded models (MCMCGPU_E_ARG). */
 #define MCMCGPU_NUTS 5
+#define MCMCGPU_NUTS_SLICE 0         /* mcmcgpu_run_set_nuts_transition */
+#define MCMCGPU_NUTS_MULTINOMIAL 1
 
 /* engines */
 #define MCMCGPU_ENGINE_AUTO 0
@@ -214,6 +220,18 @@ int32_t mcmcgpu_run_set_dense_metric(mcmcgpu_run* run, const double* inv_metric,
  * metric is Stan's unsymmetrised covariance estimate, so it need not be exactly symmetric.  MCMCGPU_E_ARG on a run
  * without a dense metric. */
 int32_t mcmcgpu_run_get_dense_metric(mcmcgpu_run* run, double* out);
+/* NUTS only, before the first execute: the transition, MCMCGPU_NUTS_SLICE (the default: a run with this call gives the
+ * bits of one without it) or MCMCGPU_NUTS_MULTINOMIAL (Stan's base_nuts transition, pinned in DESIGN.md, NUTS).  A
+ * multinomial run keeps per kept step Stan's accept_stat, the energy H of the sample and the divergence flag
+ * (mcmcgpu_run_fetch_nuts_stats); its tree state is (5 maxdoublings + 2) d + 3 maxdoublings + 2 doubles per chain, and
+ * (7 maxdoublings + 3) d + 3 maxdoublings + 2 with a dense metric.  MCMCGPU_E_ARG for another sampler or an unknown
+ * value, MCMCGPU_E_STATE after the first execute. */
+int32_t mcmcgpu_run_set_nuts_transition(mcmcgpu_run* run, int32_t transition);
+/* multinomial NUTS: per kept step (S x nchains each; any pointer may be NULL) the accept_stat (sum over the trajectory's
+ * leaves of min(1, exp(H0 - H)), over the leapfrog count), the energy H of the step's sample, and divergent = 1 when the
+ * step's last subtree stopped at a leaf with H - H0 > 1000.  MCMCGPU_E_ARG for a run that is not multinomial NUTS,
+ * MCMCGPU_E_STATE before the first execute. */
+int32_t mcmcgpu_run_fetch_nuts_stats(mcmcgpu_run* run, double* accept_stat, double* energy, uint8_t* divergent);
 int32_t mcmcgpu_run_fetch(mcmcgpu_run* run, double* out_samples, double* out_grads, uint8_t* out_accept,
                           double* out_logtarget);
 /* Rao-Blackwellised draws (store_rb): out_rb d x S x nchains; their column means are mean_rb(chain) (mean.jl:37-41) */

@@ -15,6 +15,7 @@ LIB_PATH = os.environ.get("MCMCGPU_LIB") or os.path.join(_HERE, "libmcmcgpu.so")
 OK, E_ARG, E_SUPPORT, E_NOGRAD, E_CUDA, E_COMM, E_STATE = 0, -1, -2, -3, -4, -5, -6
 FAM = dict(normal_fn=0, normal_dsl=1, linear=2, logistic=3, probit=4, ou=5, abs_normal=6)
 KIND = dict(RWM=0, MALA=1, HMC=2, HMCDA=3, RAM=4, NUTS=5)
+NUTS_SLICE, NUTS_MULTINOMIAL = 0, 1                                     # mcmcgpu_run_set_nuts_transition
 ENGINE = dict(auto=0, fused=1, wave=2)
 VTYPE = dict(iid=0, bm=1, imse=2, ipse=3)
 
@@ -59,6 +60,7 @@ EXPORTS = [
     "mcmcgpu_run_seqmc_models", "mcmcgpu_run_serialtemp_models",
     "mcmcgpu_run_set_metric", "mcmcgpu_run_set_metric_adaptation", "mcmcgpu_run_get_metric",
     "mcmcgpu_run_set_dense_metric", "mcmcgpu_run_get_dense_metric",
+    "mcmcgpu_run_set_nuts_transition", "mcmcgpu_run_fetch_nuts_stats",
 ]
 
 _lib = None
@@ -100,6 +102,8 @@ def lib():
         L.mcmcgpu_run_get_metric.argtypes = [vp, dp]
         L.mcmcgpu_run_set_dense_metric.argtypes = [vp, dp, C.c_int32]
         L.mcmcgpu_run_get_dense_metric.argtypes = [vp, dp]
+        L.mcmcgpu_run_set_nuts_transition.argtypes = [vp, C.c_int32]
+        L.mcmcgpu_run_fetch_nuts_stats.argtypes = [vp, dp, dp, C.POINTER(C.c_uint8)]
         L.mcmcgpu_run_fetch.argtypes = [vp, dp, dp, C.POINTER(C.c_uint8), dp]
         L.mcmcgpu_run_fetch_rb.argtypes = [vp, dp]
         L.mcmcgpu_run_fetch_diag.argtypes = [vp, dp, C.POINTER(C.c_int64)]
@@ -437,6 +441,17 @@ class DeviceRun(_Owned):
         out = np.empty((self.C, self.d, self.d))
         check(lib().mcmcgpu_run_get_dense_metric(self.h, dptr(out)))
         return np.ascontiguousarray(out.transpose(0, 2, 1))               # column-major blocks -> [c, i, j]
+
+    def set_nuts_transition(self, transition):
+        """NUTS, before the first execute: NUTS_SLICE (the default) or NUTS_MULTINOMIAL (Stan's transition)"""
+        check(lib().mcmcgpu_run_set_nuts_transition(self.h, int(transition)))
+
+    def fetch_nuts_stats(self):
+        """multinomial NUTS: (nchains, S) accept_stat, energy and divergent (bool) of the kept steps"""
+        acc, en = np.empty((self.C, self.S)), np.empty((self.C, self.S))
+        div = np.empty((self.C, self.S), dtype=np.uint8)
+        check(lib().mcmcgpu_run_fetch_nuts_stats(self.h, dptr(acc), dptr(en), div.ctypes.data_as(C.POINTER(C.c_uint8))))
+        return dict(accept_stat=acc, energy=en, divergent=div.astype(bool))
 
     def fetch(self, samples=True, grads=None, accept=True, logtarget=None, out=None):
         grads = self.store_grad if grads is None else grads

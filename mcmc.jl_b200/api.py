@@ -300,8 +300,13 @@ class HMCDA(_Sampler):
 
 
 class NUTS(_Sampler):
-    """No-U-Turn sampler: slice NUTS with dual averaging of the step size (Hoffman & Gelman 2014, Algorithms 3 and 6).
-    rate is the target mean acceptance statistic, maxdoublings caps the tree at 2^maxdoublings - 1 leapfrogs per step,
+    """No-U-Turn sampler with dual averaging of the step size.  transition="slice" (the default) is slice NUTS (Hoffman &
+    Gelman 2014, Algorithms 3 and 6); transition="multinomial" is Stan's transition: multinomial sampling of the
+    trajectory with biased progressive sampling between subtrees, U-turn checks across neighbouring subtrees, and per
+    kept step Stan's accept_stat, energy and divergence flag (MCMCChainBatch.nuts_stats, chain diagnostics).
+    rate is the target mean acceptance statistic (of the last doubling for slice NUTS, Stan's accept_stat over the whole
+    trajectory for multinomial NUTS; the default 0.6 is kept for both, Stan's default is 0.8), maxdoublings caps the tree
+    at 2^maxdoublings - 1 leapfrogs per step,
     shrinkage / t0 / step are the dual averaging's gamma / t0 / kappa (HMCDA's).  The mass matrix is the identity unless
     inv_metric gives a diagonal inverse metric, (d,) for every chain or (nchains, d) per chain; adapt_metric=True adapts
     each chain's diagonal metric during warm-up in Stan's windows (init_buffer / term_buffer / window, Stan's defaults),
@@ -311,13 +316,15 @@ class NUTS(_Sampler):
     model's scale is not used."""
 
     def __init__(self, rate=0.6, maxdoublings=10, shrinkage=0.05, t0=10.0, step=0.75, inv_metric=None, adapt_metric=False,
-                 init_buffer=75, term_buffer=50, window=25, metric="diag"):
+                 init_buffer=75, term_buffer=50, window=25, metric="diag", transition="slice"):
         assert 0.0 < rate < 1.0, f"Target acceptance rate ({rate}) should be between 0 and 1"
         assert isinstance(maxdoublings, (int, np.integer)) and 1 <= maxdoublings <= 10, \
             f"maxdoublings parameter of NUTS sampler ({maxdoublings}) must be an integer in 1..10"
         assert shrinkage > 0.0, f"shrinkage parameter of NUTS sampler ({shrinkage}) must be positive"
         assert t0 >= 0, f"t0 parameter of NUTS sampler ({t0}) must be non-negative"
         assert metric in ("diag", "dense"), f"metric of NUTS sampler must be 'diag' or 'dense', got {metric!r}"
+        assert transition in ("slice", "multinomial"), \
+            f"transition of NUTS sampler must be 'slice' or 'multinomial', got {transition!r}"
         if inv_metric is not None and metric == "diag":
             inv_metric = np.array(inv_metric, dtype=np.float64)
             assert inv_metric.ndim in (1, 2) and inv_metric.size > 0, \
@@ -336,12 +343,15 @@ class NUTS(_Sampler):
         for name, v, lo in (("init_buffer", init_buffer, 0), ("term_buffer", term_buffer, 0), ("window", window, 1)):
             assert isinstance(v, (int, np.integer)) and v >= lo, f"{name} of NUTS sampler ({v}) must be an integer >= {lo}"
         self.rate, self.maxdoublings, self.shrinkage, self.t0, self.step = rate, int(maxdoublings), shrinkage, t0, step
-        self.inv_metric, self.adapt_metric, self.metric = inv_metric, bool(adapt_metric), metric
+        self.inv_metric, self.adapt_metric, self.metric, self.transition = inv_metric, bool(adapt_metric), metric, transition
         self.init_buffer, self.term_buffer, self.window = int(init_buffer), int(term_buffer), int(window)
         self.tuner = None
 
     def _set_metric(self, drun, offset, nchains):
-        """the metric calls of a run of chains offset .. offset + drun.C - 1 of nchains (none with the defaults)"""
+        """the metric and transition calls of a run of chains offset .. offset + drun.C - 1 of nchains (none with the
+        defaults)"""
+        if self.transition == "multinomial":
+            drun.set_nuts_transition(capi.NUTS_MULTINOMIAL)
         if self.metric == "dense":
             m = self.inv_metric
             assert m is None or m.ndim == 2 or m.shape[0] == nchains, \
@@ -541,6 +551,8 @@ class MCMCChainBatch:
             diags["ndoublings"] = np.floor(np.log2(leaps[i])).astype(np.int64) + 1    # the tree of 2^(n-1) .. 2^n - 1 leapfrogs
             if s.inv_metric is not None or s.adapt_metric or s.metric == "dense":
                 diags["inv_metric"] = self.inv_metric()[i]
+            if s.transition == "multinomial":
+                diags.update({k: v[i] for k, v in self.nuts_stats().items()})
         g = a.get("grads")
         return MCMCChain(self.range, a["samples"][i], None if g is None else g[i], diags, self.task, self.runTime,
                          _colnames(self.task.model))
@@ -553,6 +565,13 @@ class MCMCChainBatch:
         if getattr(self, "_diag", None) is None:
             self._diag = self._run.fetch_diag()
         return self._diag
+
+    def nuts_stats(self):
+        """multinomial NUTS: dict of (C, S) arrays of the kept steps -- accept_stat (Stan's mean Metropolis acceptance over
+        the trajectory), energy (H of the draw) and divergent (bool: the last subtree stopped at H - H0 > 1000)"""
+        if getattr(self, "_nuts_stats", None) is None:
+            self._nuts_stats = self._run.fetch_nuts_stats()
+        return self._nuts_stats
 
     def inv_metric(self):
         """the inverse metric of every chain at the end of the run (NUTS): (C, d) diagonal (ones for the identity), or

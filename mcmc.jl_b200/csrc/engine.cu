@@ -109,6 +109,7 @@ struct mcmcgpu_run {
   uint8_t *need_ll = nullptr, *k1_done = nullptr;
   NutsState nuts{};          // NUTS runs only
   bool adapt_metric = false; // NUTS: mcmcgpu_run_set_metric_adaptation was called
+  bool nuts_multinomial = false;   // NUTS: mcmcgpu_run_set_nuts_transition(MCMCGPU_NUTS_MULTINOMIAL)
   int nsplit = 1;
   std::vector<void*> owned, owned_big;
   template <typename T>
@@ -674,6 +675,25 @@ __global__ void wave_init_kernel(int32_t* phase, int32_t* remaining, double* q, 
   for (int64_t j = 0; j < d; j++) q[j * Cp + c] = (c < C) ? (init_per_chain ? init[j * Cp + c] : init[j]) : 0.0;
 }
 
+// the multinomial transition's tree state and per-step outputs, at the first execute (when the metric is known)
+static int alloc_multinomial(mcmcgpu_run* R) {
+  NutsState& T = R->nuts;
+  const size_t Cp = (size_t)R->Cp, rec = (size_t)R->s.nleaps * (size_t)R->d * Cp, lev = (size_t)R->s.nleaps * Cp;
+  double** recs[] = {&T.mn_rho, &T.mn_pb, &T.mn_pe, &T.mn_th, &T.mn_g};
+  for (double** a : recs) CU(R->alloc(a, rec, false));
+  if (T.A) {
+    CU(R->alloc(&T.mn_vb, rec, false));
+    CU(R->alloc(&T.mn_ve, rec, false));
+    CU(R->alloc(&T.mn_vin, (size_t)R->d * Cp, false));
+  }
+  CU(R->alloc(&T.mn_lsw, lev, false)); CU(R->alloc(&T.mn_lt, lev, false)); CU(R->alloc(&T.mn_h, lev, false));
+  CU(R->alloc(&T.mn_trho, (size_t)R->d * Cp, false)); CU(R->alloc(&T.mn_pin, (size_t)R->d * Cp, false));
+  CU(R->alloc(&T.mn_tlsw, Cp)); CU(R->alloc(&T.mn_sh, Cp));
+  CU(R->alloc(&T.st_accept_stat, (size_t)R->S * Cp)); CU(R->alloc(&T.st_energy, (size_t)R->S * Cp));
+  CU(R->alloc(&T.st_divergent, (size_t)R->S * Cp));
+  return MCMCGPU_OK;
+}
+
 // the likelihood kernel can make the interior leapfrog updates itself when one CTA sees all rows of its chains
 static bool run_fuses_leap(const mcmcgpu_run* R) {
   const mcmcgpu_model* m = R->m;
@@ -712,6 +732,10 @@ static int execute_impl(mcmcgpu_run* R, int64_t nsteps, mcmcgpu_run_info* info) 
     launches = 1;
     R->started = true;
   } else {
+    if (R->nuts_multinomial && !R->nuts.mn_rho) {
+      int rc = alloc_multinomial(R);
+      if (rc) return rc;
+    }
     WaveArgs W;
     W.M = m->dev(); W.S = sampler_dev(R); W.R = runner_dev(R);
     const mcmcgpu_run* fuse = run_fuses_leap(R) ? R : nullptr;
@@ -1097,6 +1121,15 @@ int32_t mcmcgpu_run_get_dense_metric(mcmcgpu_run* R, double* out) {
   return MCMCGPU_OK;
 }
 
+int32_t mcmcgpu_run_set_nuts_transition(mcmcgpu_run* R, int32_t transition) {
+  if (!R) return fail(MCMCGPU_E_ARG, "run is NULL");
+  if (R->s.kind != MCMCGPU_NUTS) return fail(MCMCGPU_E_ARG, "the NUTS transition applies to NUTS");
+  if (transition != MCMCGPU_NUTS_SLICE && transition != MCMCGPU_NUTS_MULTINOMIAL) return fail(MCMCGPU_E_ARG, "unknown NUTS transition");
+  if (R->started) return fail(MCMCGPU_E_STATE, "the NUTS transition must be set before the first execute");
+  R->nuts_multinomial = transition == MCMCGPU_NUTS_MULTINOMIAL;
+  return MCMCGPU_OK;
+}
+
 int32_t mcmcgpu_run_get_state(mcmcgpu_run* R, double* pars, double* leapstep, double* dual_leapstep, double* dualH) {
   if (!R) return fail(MCMCGPU_E_ARG, "run is NULL");
   if (!R->executed) return fail(MCMCGPU_E_STATE, "run has not been executed");
@@ -1202,6 +1235,27 @@ int32_t mcmcgpu_run_fetch_diag(mcmcgpu_run* R, double* out_eps, int64_t* out_nle
     CU(cudaGetLastError());
     int rc = fetch_chunked(R, reinterpret_cast<const double*>(wide), R->S, reinterpret_cast<double*>(out_nleaps));
     if (rc) return rc;
+  }
+  return MCMCGPU_OK;
+}
+
+int32_t mcmcgpu_run_fetch_nuts_stats(mcmcgpu_run* R, double* accept_stat, double* energy, uint8_t* divergent) {
+  if (!R) return fail(MCMCGPU_E_ARG, "run is NULL");
+  if (R->s.kind != MCMCGPU_NUTS || !R->nuts_multinomial) return fail(MCMCGPU_E_ARG, "NUTS statistics are kept by multinomial NUTS runs");
+  if (!R->executed) return fail(MCMCGPU_E_STATE, "run has not been executed");
+  CU(use_ctx(R->m->ctx));
+  const NutsState& T = R->nuts;
+  int rc;
+  if (accept_stat && (rc = fetch_chunked(R, T.st_accept_stat, R->S, accept_stat))) return rc;
+  if (energy && (rc = fetch_chunked(R, T.st_energy, R->S, energy))) return rc;
+  if (divergent) {
+    cudaStream_t st = R->m->ctx->stream;
+    uint8_t* tmp = nullptr;
+    DevBufs bufs;
+    CU(bufs.get(&tmp, (size_t)(R->C * R->S), st, false));
+    CU(transpose_to_chain_major_u8(T.st_divergent, tmp, 0, R->C, R->S, R->Cp, st));
+    CU(cudaMemcpyAsync(divergent, tmp, (size_t)(R->C * R->S), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
   }
   return MCMCGPU_OK;
 }

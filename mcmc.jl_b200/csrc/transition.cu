@@ -114,7 +114,7 @@ __device__ __forceinline__ void store_kept(const WaveArgs& W, const int64_t c, i
 }
 
 // The dual-averaging update of step i < burnin (HMCDA.jl:133-138), shared by HMCDA (pacc = its acceptance probability)
-// and NUTS (pacc = the mean acceptance statistic of the step's last doubling).  The averaging counts steps from i0 and
+// and NUTS (pacc = the mean acceptance statistic of the step's last doubling, or Stan's accept_stat over the whole trajectory).  The averaging counts steps from i0 and
 // shrinks towards mu = log(ten_eps0): HMCDA passes 10 * leapStep0 (leapStep0 = 1) and i0 = 0; NUTS with metric adaptation
 // restarts it at every window end (i0 = that step, ten_eps0 = 10 eps).  The log is taken here, where HMCDA always took it,
 // so that the HMCDA kernels compile to the same instructions.
@@ -964,7 +964,122 @@ __device__ void nuts_adapt_dense(const WaveArgs& W, const int64_t c, int64_t i, 
   W.da_dual[c] = 1.0; W.da_dualH[c] = 0.0;
 }
 
+// ---- Stan's multinomial transition (base_nuts::transition / build_tree, pinned in DESIGN.md) ---------------------------
+// TR: the transition.  NUTS_TR_SLICE is the slice NUTS above; NUTS_TR_MULTI weights every leaf by exp(H0 - H), samples
+// progressively (biased at the tree level) and checks p# . rho > 0 across every pair of neighbouring blocks.  Leaf m
+// (1-based) of a subtree is written as a one-leaf block into record rf = ctz(m) -- the level at which it comes to rest, free
+// at that moment -- and merged there with the open left halves of records 0 .. rf-1 (the recursion's internal nodes it
+// closes, bottom up).  Record rf is then the left half of level rf, or for m = 2^j the finished subtree.
+constexpr int NUTS_TR_SLICE = 0, NUTS_TR_MULTI = 1;
+
+__device__ __forceinline__ double nuts_log1p_exp(double x) { return x > 0.0 ? x + log1p(exp(-x)) : log1p(exp(x)); }
+// Stan Math's log_sum_exp(a, b)
+__device__ __forceinline__ double nuts_log_sum_exp(double a, double b) {
+  if (a == -CUDART_INF) return b;
+  if (a == CUDART_INF && b == CUDART_INF) return CUDART_INF;
+  return a > b ? a + nuts_log1p_exp(b - a) : b + nuts_log1p_exp(a - b);
+}
+
+// Leaf leaf of the subtree of doubling jd (its step's 0-based leaf k) has become the tree's end on side `side` with log-weight
+// lw = H0 - h: build its block and make the merges it closes.  False when a merge finds a U-turn.
 template <int MET>
+__device__ bool nuts_mn_leaf(const WaveArgs& W, const int64_t c, const int64_t i, const uint64_t gchain, const int k, const int leaf,
+                             const int jd, const int side, double lw, double lt, double h) {
+  const NutsState& T = W.nuts;
+  const int64_t d = W.M.d, Cp = W.R.Cp, slot = d * Cp;
+  const int rf = __ffs(leaf) - 1;
+  const double* p_e = T.p[side];                                        // the leaf: p, p# (A p stored, or minv p)
+  const double* v_e = MET == NUTS_DENSE ? T.v[side] : nullptr;
+  double *rho = T.mn_rho + rf * slot, *pb = T.mn_pb + rf * slot, *th = T.mn_th + rf * slot, *g = T.mn_g + rf * slot;
+  double* vb = MET == NUTS_DENSE ? T.mn_vb + rf * slot : nullptr;
+  for (int64_t j = 0; j < d; j++) {
+    const int64_t jc = j * Cp + c;
+    const double pj = p_e[jc];
+    rho[jc] = pj; pb[jc] = pj; th[jc] = T.th[side][jc]; g[jc] = T.g[side][jc];
+    if constexpr (MET == NUTS_DENSE) vb[jc] = v_e[jc];
+  }
+  for (int r = 0; r < rf; r++) {                                        // L = record r (built first), R = record rf
+    const int64_t lo = r * slot;
+    const double lsw = nuts_log_sum_exp(T.mn_lsw[r * Cp + c], lw);
+    const bool take_r = lw > lsw ||
+        philox_slot_uniform(W.R.seed, gchain, (uint32_t)i, NUTS_LEAF_BLOCK + (uint32_t)(k - (1 << r))) < exp(lw - lsw);
+    double a1 = 0.0, b1 = 0.0, a2 = 0.0, b2 = 0.0, a3 = 0.0, b3 = 0.0;
+    for (int64_t j = 0; j < d; j++) {
+      const int64_t jc = j * Cp + c;
+      const double rl = T.mn_rho[lo + jc], rr = rho[jc], pbl = T.mn_pb[lo + jc], pel = T.mn_pe[lo + jc], pbr = pb[jc];
+      double sbl, sel, sbr, se;
+      if constexpr (MET == NUTS_DENSE) {
+        sbl = T.mn_vb[lo + jc]; sel = T.mn_ve[lo + jc]; sbr = vb[jc]; se = v_e[jc];
+      } else {
+        sbl = nuts_mv<MET == NUTS_DIAG>(T.minv, jc, pbl); sel = nuts_mv<MET == NUTS_DIAG>(T.minv, jc, pel);
+        sbr = nuts_mv<MET == NUTS_DIAG>(T.minv, jc, pbr); se = nuts_mv<MET == NUTS_DIAG>(T.minv, jc, p_e[jc]);
+      }
+      const double rs = rl + rr, x = rl + pbr, y = rr + pel;
+      a1 += sbl * rs; b1 += se * rs;                                    // crit(p#[beg L], p#[end R], rho)
+      a2 += sbl * x; b2 += sbr * x;                                     // crit(p#[beg L], p#[beg R], rho_L + p[beg R])
+      a3 += sel * y; b3 += se * y;                                      // crit(p#[end L], p#[end R], rho_R + p[end L])
+      rho[jc] = rs; pb[jc] = pbl;
+      if constexpr (MET == NUTS_DENSE) vb[jc] = sbl;
+      if (!take_r) { th[jc] = T.mn_th[lo + jc]; g[jc] = T.mn_g[lo + jc]; }
+    }
+    if (!take_r) { lt = T.mn_lt[r * Cp + c]; h = T.mn_h[r * Cp + c]; }
+    lw = lsw;
+    if (!(a1 > 0.0 && b1 > 0.0 && a2 > 0.0 && b2 > 0.0 && a3 > 0.0 && b3 > 0.0)) return false;
+  }
+  T.mn_lsw[rf * Cp + c] = lw; T.mn_lt[rf * Cp + c] = lt; T.mn_h[rf * Cp + c] = h;
+  if (rf < jd)                                                          // a left half: keep its last-built leaf
+    for (int64_t j = 0; j < d; j++) {
+      const int64_t jc = j * Cp + c;
+      T.mn_pe[rf * slot + jc] = p_e[jc];
+      if constexpr (MET == NUTS_DENSE) T.mn_ve[rf * slot + jc] = v_e[jc];
+    }
+  return true;
+}
+
+// The subtree of doubling jd (record jd) is complete and valid: biased progressive sampling of the step's sample, the tree's
+// log-sum-weight, and (when another doubling is allowed) the U-turn checks of the merged tree, which is B (backward) + F
+// (forward): the old tree and the subtree by side.  Returns whether the tree goes on.
+template <int MET>
+__device__ bool nuts_mn_tree(const WaveArgs& W, const int64_t c, const int64_t i, const uint64_t gchain, const int jd, const int side) {
+  const NutsState& T = W.nuts;
+  const int64_t d = W.M.d, Cp = W.R.Cp, so = jd * W.M.d * W.R.Cp;
+  const double lsw_s = T.mn_lsw[jd * Cp + c], lsw_t = T.mn_tlsw[c];
+  if (lsw_s > lsw_t ||
+      philox_slot_uniform(W.R.seed, gchain, (uint32_t)i, NUTS_TREE_BLOCK + 2u * (uint32_t)jd + 1u) < exp(lsw_s - lsw_t)) {
+    for (int64_t j = 0; j < d; j++) { W.cur_pars[j * Cp + c] = T.mn_th[so + j * Cp + c]; W.cur_grad[j * Cp + c] = T.mn_g[so + j * Cp + c]; }
+    W.cur_lt[c] = T.mn_lt[jd * Cp + c]; T.mn_sh[c] = T.mn_h[jd * Cp + c];
+    T.moved[c] = 1;
+  }
+  T.mn_tlsw[c] = nuts_log_sum_exp(lsw_t, lsw_s);
+  if (jd + 1 >= W.S.nleaps) return false;
+  // B- and F+ are the tree's ends; B+ / F- are the old tree's inner end and the subtree's first leaf, by side
+  const double* pbp = side ? T.mn_pin : T.mn_pb + so;
+  const double* pfm = side ? T.mn_pb + so : T.mn_pin;
+  const double* vbp = MET == NUTS_DENSE ? (side ? T.mn_vin : T.mn_vb + so) : nullptr;
+  const double* vfm = MET == NUTS_DENSE ? (side ? T.mn_vb + so : T.mn_vin) : nullptr;
+  const double* rho_b = side ? T.mn_trho : T.mn_rho + so;
+  const double* rho_f = side ? T.mn_rho + so : T.mn_trho;
+  double a1 = 0.0, b1 = 0.0, a2 = 0.0, b2 = 0.0, a3 = 0.0, b3 = 0.0;
+  for (int64_t j = 0; j < d; j++) {
+    const int64_t jc = j * Cp + c;
+    const double rb = rho_b[jc], rf = rho_f[jc], pb_p = pbp[jc], pf_m = pfm[jc];
+    double sbm, sfp, sbp, sfm;
+    if constexpr (MET == NUTS_DENSE) {
+      sbm = T.v[0][jc]; sfp = T.v[1][jc]; sbp = vbp[jc]; sfm = vfm[jc];
+    } else {
+      sbm = nuts_mv<MET == NUTS_DIAG>(T.minv, jc, T.p[0][jc]); sfp = nuts_mv<MET == NUTS_DIAG>(T.minv, jc, T.p[1][jc]);
+      sbp = nuts_mv<MET == NUTS_DIAG>(T.minv, jc, pb_p); sfm = nuts_mv<MET == NUTS_DIAG>(T.minv, jc, pf_m);
+    }
+    const double rs = rb + rf, x = rb + pf_m, y = rf + pb_p;
+    a1 += sbm * rs; b1 += sfp * rs;                                     // crit(p#[B-], p#[F+], rho)
+    a2 += sbm * x; b2 += sfm * x;                                       // crit(p#[B-], p#[F-], rho_B + p[F-])
+    a3 += sbp * y; b3 += sfp * y;                                       // crit(p#[B+], p#[F+], rho_F + p[B+])
+    T.mn_trho[jc] = rs;
+  }
+  return a1 > 0.0 && b1 > 0.0 && a2 > 0.0 && b2 > 0.0 && a3 > 0.0 && b3 > 0.0;
+}
+
+template <int MET, int TR>
 __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
   const RunnerDev& R = W.R;
   const SamplerDev& S = W.S;
@@ -1031,31 +1146,42 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       }
     const double* w_v = MET == NUTS_DENSE ? T.v[side] : p_v;            // what the U-turn dots take: A p, or p
     const double H = -F.lt + 0.5 * mm;                                  // update! HMC.jl:91
-    const double H0 = W.H0[c], lu0 = T.log_u0[c];
+    const double H0 = W.H0[c], lu0 = TR == NUTS_TR_SLICE ? T.log_u0[c] : 0.0;
     const int k = T.leaps[c];
     T.leaps[c] = k + 1;
-    const double ea = exp(H0 - H);
-    const double alpha = T.alpha[c] + (isnan(ea) ? 0.0 : (ea < 1.0 ? ea : 1.0));
-    T.alpha[c] = alpha;
-    bool s = H - H0 < 1000.0 - lu0;                                     // false for NaN
-    if (lu0 <= H0 - H) {                                                // a valid leaf: candidate with probability 1 / n_sub
-      const int nsub = T.n_sub[c] + 1;
-      T.n_sub[c] = nsub;
-      if (nsub == 1 || philox_slot_uniform(R.seed, gchain, (uint32_t)i, NUTS_LEAF_BLOCK + (uint32_t)k) * (double)nsub < 1.0) {
-        for (int64_t j = 0; j < d; j++) { T.sub_pars[j * Cp + c] = th_v[j * Cp + c]; T.sub_grad[j * Cp + c] = g_v[j * Cp + c]; }
-        T.sub_lt[c] = F.lt;
+    double alpha;
+    bool s, divergent = false;
+    if constexpr (TR == NUTS_TR_SLICE) {
+      const double ea = exp(H0 - H);
+      alpha = T.alpha[c] + (isnan(ea) ? 0.0 : (ea < 1.0 ? ea : 1.0));
+      T.alpha[c] = alpha;
+      s = H - H0 < 1000.0 - lu0;                                        // false for NaN
+      if (lu0 <= H0 - H) {                                              // a valid leaf: candidate with probability 1 / n_sub
+        const int nsub = T.n_sub[c] + 1;
+        T.n_sub[c] = nsub;
+        if (nsub == 1 || philox_slot_uniform(R.seed, gchain, (uint32_t)i, NUTS_LEAF_BLOCK + (uint32_t)k) * (double)nsub < 1.0) {
+          for (int64_t j = 0; j < d; j++) { T.sub_pars[j * Cp + c] = th_v[j * Cp + c]; T.sub_grad[j * Cp + c] = g_v[j * Cp + c]; }
+          T.sub_lt[c] = F.lt;
+        }
       }
+      const int64_t slot = d * Cp;
+      for (int r = 1; s && r <= jd && (leaf & ((1 << r) - 1)) == 0; r++)      // U-turn checks of the blocks this leaf closes
+        s = nuts_no_uturn<MET == NUTS_DIAG>(th_v, w_v, T.ck_th + (r - 1) * slot, T.ck_p + (r - 1) * slot, v, T.minv, d, Cp, c);
+    } else {                                                            // Stan's leaf: h, divergence, sum_metro, its block
+      const double h = isnan(H) ? CUDART_INF : H;
+      divergent = h - H0 > 1000.0;
+      alpha = T.alpha[c] + (H0 - h > 0.0 ? 1.0 : exp(H0 - h));
+      T.alpha[c] = alpha;
+      s = !divergent && nuts_mn_leaf<MET>(W, c, i, gchain, k, leaf, jd, side, H0 - h, F.lt, h);
     }
-    const int64_t slot = d * Cp;
-    for (int r = 1; s && r <= jd && (leaf & ((1 << r) - 1)) == 0; r++)        // U-turn checks of the blocks this leaf closes
-      s = nuts_no_uturn<MET == NUTS_DIAG>(th_v, w_v, T.ck_th + (r - 1) * slot, T.ck_p + (r - 1) * slot, v, T.minv, d, Cp, c);
     bool open = false;
     if (s && leaf < (1 << jd)) {                                        // next leaf of this subtree
-      for (int r = 1; r <= jd && ((leaf - 1) & ((1 << r) - 1)) == 0; r++)     // checkpoints of the blocks this leaf opens
-        for (int64_t j = 0; j < d; j++) {
-          T.ck_th[(r - 1) * slot + j * Cp + c] = th_v[j * Cp + c];
-          T.ck_p[(r - 1) * slot + j * Cp + c] = w_v[j * Cp + c];
-        }
+      if constexpr (TR == NUTS_TR_SLICE)
+        for (int r = 1; r <= jd && ((leaf - 1) & ((1 << r) - 1)) == 0; r++)   // checkpoints of the blocks this leaf opens
+          for (int64_t j = 0, slot = d * Cp; j < d; j++) {
+            T.ck_th[(r - 1) * slot + j * Cp + c] = th_v[j * Cp + c];
+            T.ck_p[(r - 1) * slot + j * Cp + c] = w_v[j * Cp + c];
+          }
       for (int64_t j = 0; j < d; j++) {                                 // HMC.jl:95-96 from the end just reached
         double m = p_v[j * Cp + c];
         m += (0.5 * g_v[j * Cp + c]) * e;
@@ -1071,20 +1197,30 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
       T.leaf[c] = leaf + 1;
       return nev;
     } else if (s) {                                                     // the subtree is complete: merge it into the tree
-      const int n = T.n[c], nsub = T.n_sub[c];
-      if (philox_slot_uniform(R.seed, gchain, (uint32_t)i, NUTS_TREE_BLOCK + 2u * (uint32_t)jd + 1u) * (double)n < (double)nsub) {
-        for (int64_t j = 0; j < d; j++) { W.cur_pars[j * Cp + c] = T.sub_pars[j * Cp + c]; W.cur_grad[j * Cp + c] = T.sub_grad[j * Cp + c]; }
-        W.cur_lt[c] = T.sub_lt[c];
-        T.moved[c] = 1;
+      if constexpr (TR == NUTS_TR_SLICE) {
+        const int n = T.n[c], nsub = T.n_sub[c];
+        if (philox_slot_uniform(R.seed, gchain, (uint32_t)i, NUTS_TREE_BLOCK + 2u * (uint32_t)jd + 1u) * (double)n < (double)nsub) {
+          for (int64_t j = 0; j < d; j++) { W.cur_pars[j * Cp + c] = T.sub_pars[j * Cp + c]; W.cur_grad[j * Cp + c] = T.sub_grad[j * Cp + c]; }
+          W.cur_lt[c] = T.sub_lt[c];
+          T.moved[c] = 1;
+        }
+        T.n[c] = n + nsub;
+        open = jd + 1 < S.nleaps && nuts_no_uturn<MET == NUTS_DIAG>(T.th[1], MET == NUTS_DENSE ? T.v[1] : T.p[1], T.th[0],
+                                                                     MET == NUTS_DENSE ? T.v[0] : T.p[0], 1.0, T.minv, d, Cp, c);
+      } else {
+        open = nuts_mn_tree<MET>(W, c, i, gchain, jd, side);
       }
-      T.n[c] = n + nsub;
-      open = jd + 1 < S.nleaps && nuts_no_uturn<MET == NUTS_DIAG>(T.th[1], MET == NUTS_DENSE ? T.v[1] : T.p[1], T.th[0],
-                                                                   MET == NUTS_DENSE ? T.v[0] : T.p[0], 1.0, T.minv, d, Cp, c);
     }
     if (open) {
       doubling = true; jnext = jd + 1;
     } else {                                                            // the tree is closed: the step's sample is final
-      const double pacc = alpha / (double)leaf;                         // alpha / n_alpha of the last doubling
+      // slice: alpha / n_alpha of the last doubling; multinomial: sum_metro / n_leapfrog of the step
+      const double pacc = alpha / (double)(TR == NUTS_TR_SLICE ? leaf : k + 1);
+      if constexpr (TR == NUTS_TR_MULTI)
+        if (in_range(i, R.first, R.step, R.last)) {
+          const int64_t kk = W.kept[c];
+          T.st_accept_stat[kk * Cp + c] = pacc; T.st_energy[kk * Cp + c] = T.mn_sh[c]; T.st_divergent[kk * Cp + c] = divergent ? 1 : 0;
+        }
       store_kept(W, c, i, true, T.moved[c] != 0, W.eps_cur[c], k + 1);
       if (i < burnin) {
         double eps0 = 1.0;
@@ -1130,6 +1266,7 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
         T.th[0][j * Cp + c] = pj; T.th[1][j * Cp + c] = pj;
         T.p[0][j * Cp + c] = z; T.p[1][j * Cp + c] = z;
         T.g[0][j * Cp + c] = gj; T.g[1][j * Cp + c] = gj;
+        if constexpr (TR == NUTS_TR_MULTI && MET != NUTS_DENSE) T.mn_trho[j * Cp + c] = z;
       }
     }
     if constexpr (MET == NUTS_DENSE) {   // p = L^-T z by back substitution (Stan's llt().matrixU().solve), v = A p, K = 0.5 v . p
@@ -1145,17 +1282,29 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
         const double vj = dense_row(T.A + (T.a_ld == 1 ? 0 : c), T.a_ld, j, p0, d, Cp, c);
         mm += vj * pj;
         T.p[1][j * Cp + c] = pj; T.v[0][j * Cp + c] = vj; T.v[1][j * Cp + c] = vj;
+        if constexpr (TR == NUTS_TR_MULTI) T.mn_trho[j * Cp + c] = pj;
       }
     }
     W.H0[c] = -W.cur_lt[c] + 0.5 * mm;                                  // update! HMC.jl:91
-    T.log_u0[c] = log(philox_uniform(R.seed, gchain, (uint32_t)i));
-    T.n[c] = 1; T.leaps[c] = 0; T.moved[c] = 0;
+    if constexpr (TR == NUTS_TR_SLICE) {
+      T.log_u0[c] = log(philox_uniform(R.seed, gchain, (uint32_t)i));
+      T.n[c] = 1;
+    } else {                                                            // the one-point tree: log-weight 0, sample H = H0
+      T.mn_tlsw[c] = 0.0; T.mn_sh[c] = W.H0[c]; T.alpha[c] = 0.0;
+    }
+    T.leaps[c] = 0; T.moved[c] = 0;
     W.eps_cur[c] = W.da_leapstep[c];
     doubling = true; jnext = 0;
   }
   if (doubling) {   // doubling jnext: direction, then the first leaf of its subtree from the end on that side
     const int side = philox_slot_uniform(R.seed, gchain, (uint32_t)i, NUTS_TREE_BLOCK + 2u * (uint32_t)jnext) >= 0.5 ? 1 : 0;
-    T.j[c] = jnext; T.dir[c] = side; T.leaf[c] = 1; T.n_sub[c] = 0; T.alpha[c] = 0.0;
+    T.j[c] = jnext; T.dir[c] = side; T.leaf[c] = 1;
+    if constexpr (TR == NUTS_TR_SLICE) { T.n_sub[c] = 0; T.alpha[c] = 0.0; }
+    else                                                                // the old tree's end on this side becomes its inner end
+      for (int64_t j = 0; j < d; j++) {
+        T.mn_pin[j * Cp + c] = T.p[side][j * Cp + c];
+        if constexpr (MET == NUTS_DENSE) T.mn_vin[j * Cp + c] = T.v[side][j * Cp + c];
+      }
     const double e = (side ? 1.0 : -1.0) * W.eps_cur[c];
     const double* th_v = T.th[side];
     const double* p_v = T.p[side];
@@ -1179,11 +1328,11 @@ __device__ int nuts_chain(const WaveArgs& W, const int64_t c) {
 }
 
 constexpr int NUTS_THREADS = 128;
-template <int MET>
+template <int MET, int TR>
 __global__ void __launch_bounds__(NUTS_THREADS) nuts_kernel(const WaveArgs W) {
   if (!W.resume && *W.remaining == 0) return;
   const int64_t c = (int64_t)blockIdx.x * NUTS_THREADS + threadIdx.x;
-  const int nev = (c < W.R.C) ? nuts_chain<MET>(W, c) : 0;
+  const int nev = (c < W.R.C) ? nuts_chain<MET, TR>(W, c) : 0;
   const int total = __syncthreads_count(nev);
   if (threadIdx.x == 0 && total) atomicAdd(W.n_evals, (unsigned long long)total);
 }
@@ -1191,9 +1340,13 @@ __global__ void __launch_bounds__(NUTS_THREADS) nuts_kernel(const WaveArgs W) {
 cudaError_t launch_transition(const WaveArgs& W, cudaStream_t st) {
   if (W.S.kind == MCMCGPU_NUTS) {
     const unsigned blocks = (unsigned)((W.R.C + NUTS_THREADS - 1) / NUTS_THREADS);
-    if (W.nuts.A) nuts_kernel<NUTS_DENSE><<<blocks, NUTS_THREADS, 0, st>>>(W);
-    else if (W.nuts.minv) nuts_kernel<NUTS_DIAG><<<blocks, NUTS_THREADS, 0, st>>>(W);
-    else nuts_kernel<NUTS_UNIT><<<blocks, NUTS_THREADS, 0, st>>>(W);
+    if (W.nuts.mn_rho) {
+      if (W.nuts.A) nuts_kernel<NUTS_DENSE, NUTS_TR_MULTI><<<blocks, NUTS_THREADS, 0, st>>>(W);
+      else if (W.nuts.minv) nuts_kernel<NUTS_DIAG, NUTS_TR_MULTI><<<blocks, NUTS_THREADS, 0, st>>>(W);
+      else nuts_kernel<NUTS_UNIT, NUTS_TR_MULTI><<<blocks, NUTS_THREADS, 0, st>>>(W);
+    } else if (W.nuts.A) nuts_kernel<NUTS_DENSE, NUTS_TR_SLICE><<<blocks, NUTS_THREADS, 0, st>>>(W);
+    else if (W.nuts.minv) nuts_kernel<NUTS_DIAG, NUTS_TR_SLICE><<<blocks, NUTS_THREADS, 0, st>>>(W);
+    else nuts_kernel<NUTS_UNIT, NUTS_TR_SLICE><<<blocks, NUTS_THREADS, 0, st>>>(W);
     return cudaGetLastError();
   }
   const bool regression = (W.M.family == MCMCGPU_FAM_LINEAR || W.M.family == MCMCGPU_FAM_LOGISTIC || W.M.family == MCMCGPU_FAM_PROBIT);

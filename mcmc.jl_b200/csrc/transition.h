@@ -44,6 +44,17 @@ struct NutsState {
   double* L;                   // lower Cholesky factor of A (the upper triangle is not used)
   double* v[2];                // [d][Cp] A p of each tree end; with a dense metric ck_p holds A p instead of p
   int64_t a_ld;
+  // Stan's multinomial transition (mcmcgpu_run_set_nuts_transition; null mn_rho: slice NUTS).  Block records, one per level
+  // r = 0 .. maxdoublings-1, each [maxdoublings][d][Cp]: record r holds the open left half of 2^r leaves of the subtree being
+  // built, and record j the finished subtree of doubling j.  A block keeps the sum of its momenta, the momentum p of its
+  // first- and last-built leaves (pb, pe), its proposal (theta, grad) and, with a dense metric, A p of both end leaves (vb,
+  // ve); p# = minv p is recomputed for the identity and diagonal metrics.  alpha sums the Metropolis statistic over the step.
+  double *mn_rho, *mn_pb, *mn_pe, *mn_th, *mn_g, *mn_vb, *mn_ve;
+  double *mn_lsw, *mn_lt, *mn_h;        // [maxdoublings][Cp] log-sum-weight, proposal's log-target and H
+  double *mn_trho, *mn_pin, *mn_vin;    // [d][Cp] the tree's momentum sum; p (A p) of the old tree's end on the growing side
+  double *mn_tlsw, *mn_sh;              // [Cp] the tree's log-sum-weight; H of the step's sample
+  double *st_accept_stat, *st_energy;   // [S][Cp] per kept step: sum_metro / n_leapfrog, H of the sample
+  uint8_t* st_divergent;                // [S][Cp] the step's last subtree stopped at a divergent leaf
 };
 
 struct WaveArgs {

@@ -84,7 +84,11 @@ samplercfg(s::NUTS)  = SamplerCfg(5, s.maxdoublings, 0., s.rate, 0., s.shrinkage
 #   invmetric::Union(Nothing, Array{Float64})   # d, or d x nchains; nothing = the identity
 #   adaptmetric::Bool; initbuffer::Int; termbuffer::Int; window::Int   # Stan's windows, defaults 75 / 50 / 25
 #   metric::Symbol                              # :diag, or :dense with invmetric d x d / d x d x nchains (nothing = I)
+#   transition::Symbol                          # :slice (default), or :multinomial (Stan's transition)
 function nuts_metric!(run::Ptr{Void}, s::NUTS)
+  if s.transition == :multinomial
+    check(ccall((:mcmcgpu_run_set_nuts_transition, libmcmcgpu), Int32, (Ptr{Void}, Int32), run, 1))
+  end
   if s.metric == :dense
     check(ccall((:mcmcgpu_run_set_dense_metric, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}, Int32),
                 run, s.invmetric == nothing ? C_NULL : s.invmetric, s.invmetric != nothing && ndims(s.invmetric) == 3 ? 1 : 0))
@@ -108,6 +112,14 @@ function nuts_dense_metric(run::Ptr{Void}, d::Int, nchains::Int)
   out = Array(Float64, d, d, nchains)
   check(ccall((:mcmcgpu_run_get_dense_metric, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}), run, out))
   out
+end
+
+# multinomial NUTS: the accept_stat, energy and divergence flag of every kept step, S x nchains each
+function nuts_stats(run::Ptr{Void}, S::Int, nchains::Int)
+  acc, energy, div = Array(Float64, S, nchains), Array(Float64, S, nchains), Array(UInt8, S, nchains)
+  check(ccall((:mcmcgpu_run_fetch_nuts_stats, libmcmcgpu), Int32, (Ptr{Void}, Ptr{Float64}, Ptr{Float64}, Ptr{UInt8}),
+              run, acc, energy, div))
+  acc, energy, div .!= 0
 end
 
 function run_gpumc(t::MCMCTask)
